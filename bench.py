@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Nexmark events/s through the B200 Z-set hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--query q3|q4|q7]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--query q3|q4|q7] [--dump-outputs DIR]
 
 Workload.  A *circuit step* is one `Circuit::step()` of the query over E = 5 M synthetic Nexmark events per
 GPU.  A *bench step* (what --steps / --warmup count) is S consecutive circuit steps (S per query below), so that
@@ -22,6 +22,12 @@ the config[4] merge sweep ride along under `queries` / `merge_sweep` unless --qu
              between steps (the Rust reference cannot be built here: no rustc), rebuilt with -march=native on the box
              it is timed on.  `--impl reference` runs the SAME circuit steps as the GPU arm (same E, same S, same
              K and W); the in-line `cpu_baseline` of a default run is a bounded sample (fewer steps, stated).
+`--dump-outputs DIR`: after the timed steps, the primary query's output Z-set of the last timed circuit step goes to
+             DIR as float64 .npy files (see dump_outputs), so that two builds run with the same arguments (hence the
+             same seeded inputs) can be compared output for output.
+
+bench.py writes nothing into the source tree (which may be read-only): the CPU arm's -march=native build goes to a
+temporary directory and no bytecode is cached.
 """
 from __future__ import annotations
 
@@ -36,6 +42,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+DUMP_LIMIT_BYTES = 64 << 20
 
 METRIC = "nexmark_events_per_sec"
 UNIT = "events/s"
@@ -166,8 +173,38 @@ def workload_cfg(query, E, S, W, K, world):
     return cfg
 
 
-def run_b200(args, query, rank, world, comm, device, do_e2e=True):
-    """Returns dict with value / e2e / profile for `query` on this rank."""
+def flat_rows(batch):
+    """A batch's rows as flat uint64 lanes (keys, then values) and int64 weights, in the batch's canonical order."""
+    d = batch.download()
+    lanes = [np.asarray(k).view(np.uint64) for k in d["keys"]]
+    if d["offs"] is not None:
+        counts = np.diff(d["offs"].astype(np.int64))
+        lanes = [np.repeat(k, counts) for k in lanes] + [np.asarray(v).view(np.uint64) for v in d["vals"]]
+    return lanes, d["diffs"]
+
+
+def dump_outputs(out_dir, prefix, lanes, weights, limit_bytes):
+    """Writes one output Z-set as float64 .npy files: every uint64 lane as its two 32-bit halves
+    (`<prefix>lane<i>_hi`, `<prefix>lane<i>_lo`; float64 holds them exactly) and `<prefix>weight`.  An output larger
+    than `limit_bytes` is cut to a fixed, seeded sample of rows whose indices go to `<prefix>row_index`."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+    row_bytes = 8 * (2 * len(lanes) + 2)
+    if len(weights) * row_bytes > limit_bytes:
+        idx = np.sort(np.random.default_rng(0).choice(len(weights), limit_bytes // row_bytes, replace=False))
+        lanes, weights = [c[idx] for c in lanes], weights[idx]
+        arrays["row_index"] = idx
+    for i, c in enumerate(lanes):
+        arrays[f"lane{i}_hi"] = c >> np.uint64(32)
+        arrays[f"lane{i}_lo"] = c & np.uint64(0xFFFFFFFF)
+    arrays["weight"] = weights
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), a.astype(np.float64))
+
+
+def run_b200(args, query, rank, world, comm, device, do_e2e=True, keep_output=False):
+    """Returns dict with value / e2e / profile for `query` on this rank; with keep_output, also `output`: the flat
+    rows of the last timed circuit step's output Z-set."""
     import torch
 
     import dbsp_b200
@@ -249,6 +286,8 @@ def run_b200(args, query, rank, world, comm, device, do_e2e=True):
     prof = be.profile_read()
     be.profile(False)
     out_rows = len(out.value)
+    if keep_output:
+        res["output"] = flat_rows(out.value)
     in_rows = rows_in(steps, W, W + K)
     res.update(value=world * E * K / (ms / 1e3), rows_per_s=world * in_rows / (ms / 1e3), ms_per_step=ms / args.steps,
                ms_per_circuit_step=ms / K, wall_ms_per_circuit_step=wall * 1e3 / K,
@@ -521,6 +560,7 @@ def run_reference(args, query, bench_steps=None, warmup=None, n_workers=None, gp
 
 
 def main():
+    sys.dont_write_bytecode = True   # no __pycache__ of the in-tree modules the runs import
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=20)
@@ -532,7 +572,11 @@ def main():
     ap.add_argument("--cpu-threads", type=int, default=16)
     ap.add_argument("--no-extras", action="store_true", help="skip q4/q7, the merge sweep and the in-line cpu_baseline")
     ap.add_argument("--sweep-rows", default="10000000,100000000,1000000000", help="config[4] total rows per merge")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the primary query's output of the last timed circuit step to DIR as .npy files")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the GPU arm: the CPU arm returns only a fingerprint per step")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -578,7 +622,10 @@ def main():
         dist.init_process_group("nccl", device_id=device)
         comm = make_comm(device)
 
-    res = run_b200(args, primary, rank, world, comm, device)
+    res = run_b200(args, primary, rank, world, comm, device, keep_output=bool(args.dump_outputs))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, f"{primary}_" if world == 1 else f"{primary}_rank{rank}_", *res.pop("output"),
+                     limit_bytes=DUMP_LIMIT_BYTES // world)
     cfg = workload_cfg(primary, E, S, W, K, world)
     line = {"metric": METRIC, "value": res["value"], "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
             "ms_per_step": res["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,

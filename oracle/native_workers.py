@@ -8,24 +8,30 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 QUERY_ID = {"q3": 3, "q4": 4, "q7": 7}
 _libs = {}
+_tmpdirs = []   # keeps the native build's directory alive while its library is loaded
 
 
 def load(native: bool = False):
-    """native=True: rebuild with -march=native on THIS machine (oracle/native/); falls back to the portable build."""
+    """native=True: rebuild with -march=native on THIS machine, into a temporary directory removed at exit (the
+    source tree may be read-only); falls back to the portable build."""
     key = "native" if native else "portable"
     if key in _libs:
         return _libs[key]
     path, how = os.path.join(HERE, "liborc_workers.so"), "portable (-O3)"
     if native:
         try:
-            subprocess.check_call(["make", "-C", HERE, "native", "-s"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
-            path, how = os.path.join(HERE, "native", "liborc_workers.so"), "-O3 -march=native, built on this host"
+            out = tempfile.TemporaryDirectory(prefix="dbsp_orc_native_")
+            _tmpdirs.append(out)
+            subprocess.check_call(["make", "-C", HERE, "native", f"NATIVE={out.name}", "-s"],
+                                  stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            path, how = os.path.join(out.name, "liborc_workers.so"), "-O3 -march=native, built on this host"
         except Exception:
             pass
     if not os.path.exists(path):

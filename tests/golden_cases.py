@@ -483,5 +483,5 @@ def run_window_bounded_memory(be, steps=1500):
     assert len(out.value) <= 200
 
 
-# written after the round's GPU budget ended: the oracle runs it; its CUDA twin is a non-strict xfail (test_zz_gpu_late.py)
+# run on the oracle by test_oracle_golden.py and on the CUDA library by test_zz_gpu_late.py
 ORACLE_ONLY_CASES = {"window_bounded_memory": run_window_bounded_memory}

@@ -5,6 +5,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -59,3 +62,64 @@ def test_reference_arm_bounded_sample_is_declared():
 def test_gpu_arm_refuses_without_device():
     rc, d = run_bench("--steps", "1", env={"CUDA_VISIBLE_DEVICES": ""})
     assert rc != 0 and "no CUDA device" in d["error"]
+
+
+def load_dump(d, prefix, n_lanes):
+    """(lanes, weights, row indices or None) of a --dump-outputs directory, lanes reassembled from their halves."""
+    lanes = [(np.load(os.path.join(d, f"{prefix}lane{i}_hi.npy")).astype(np.uint64) << np.uint64(32))
+             | np.load(os.path.join(d, f"{prefix}lane{i}_lo.npy")).astype(np.uint64) for i in range(n_lanes)]
+    idx = os.path.join(d, f"{prefix}row_index.npy")
+    return lanes, np.load(os.path.join(d, f"{prefix}weight.npy")), (np.load(idx).astype(np.int64) if os.path.exists(idx) else None)
+
+
+@pytest.mark.parametrize("limit", [64 << 20, 8 * 8 * 100], ids=["whole", "sampled"])
+def test_dump_outputs_exact_and_bounded(tmp_path, oracle, limit):
+    # lanes above 2**53 must survive the float64 files bit for bit; an output over the limit becomes a seeded sample
+    sys.path.insert(0, ROOT)
+    import bench
+    import dbsp_b200
+
+    rng = np.random.default_rng(3)
+    b = oracle.batch_from_columns(dbsp_b200.Schema("u", "uu"), [rng.integers(0, 50, 4000).astype(np.uint64),
+                                  rng.integers(0, 1 << 62, 4000).astype(np.uint64), rng.integers(0, 9, 4000).astype(np.uint64)],
+                                  rng.integers(-2, 3, 4000))
+    lanes, w = bench.flat_rows(b)
+    ref_lanes, ref_w = oracle.flat(b)
+    assert all(np.array_equal(x, y) for x, y in zip(lanes, ref_lanes)) and np.array_equal(w, ref_w)
+    for d in (tmp_path / "a", tmp_path / "b"):
+        bench.dump_outputs(str(d), "q_", lanes, w, limit)
+    got, gw, idx = load_dump(tmp_path / "a", "q_", 3)
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= limit + 8 * 128   # + the .npy headers
+    if limit == 64 << 20:
+        assert idx is None
+        idx = np.arange(len(w))
+    else:
+        assert len(idx) == 100 and np.all(np.diff(idx) > 0)
+        assert np.array_equal(idx, load_dump(tmp_path / "b", "q_", 3)[2])
+    assert all(np.array_equal(g, c[idx]) for g, c in zip(got, lanes)) and np.array_equal(gw, w[idx].astype(np.float64))
+
+
+@pytest.mark.gpu
+def test_gpu_dump_outputs_match_oracle(tmp_path, oracle):
+    # --steps K times K bench steps, and --dump-outputs holds the output of the last of them: the oracle circuit fed
+    # the same seeded warm-up + timed circuit steps ends on the same Z-set
+    sys.path.insert(0, ROOT)
+    import bench
+    import dbsp_b200
+    from dbsp_b200.nexmark import queries as nq
+
+    E, W, K = 100_000, 3, 2
+    rc, d = run_bench("--query", "q3", "--no-extras", "--steps", str(K), "--warmup", str(W), "--circuit-steps", "1",
+                      "--events-per-step", str(E), "--dump-outputs", str(tmp_path))
+    assert rc == 0 and d["steps"] == K and d["config"]["timed_circuit_steps"] == K
+    c = dbsp_b200.RootCircuit(oracle, None)
+    inp, handles = nq.add_nexmark_input(c)
+    out = nq.QUERIES["q3"](inp).output()
+    for t in bench.gen_steps("q3", 0, 1, W + K, E, pinned=False):
+        for k in ("person", "auction", "bid"):
+            handles[k].set(t[k] if t[k] is not None else bench.empty_cols())
+        c.step()
+    lanes, w = bench.flat_rows(out.value)
+    got, gw, idx = load_dump(tmp_path, "q3_", len(lanes))
+    assert len(w) > 0 and idx is None
+    assert all(np.array_equal(g, x) for g, x in zip(got, lanes)) and np.array_equal(gw, w.astype(np.float64))

@@ -1,14 +1,12 @@
-"""CUDA twins of the golden cases that were transcribed after the round's GPU budget ended (their oracle twins run
-under `-m "not gpu"`): filter_map_test, index_test / index_with_test, zset_sum, propagate_test, window bounded_memory.
-They have never run on a GPU, so they are non-strict xfail — an unrun test must not be able to turn the suite red —
-and this file sorts last so that nothing runs after them.  Expected outcome: XPASS."""
+"""CUDA twins of the later golden cases (their oracle twins run under `-m "not gpu"`): filter_map_test,
+index_test / index_with_test, zset_sum, propagate_test, window bounded_memory."""
 import pytest
 
 import filter_map_cases as fc
 import golden_cases as gc
 import recursion_cases as rc
 
-pytestmark = [pytest.mark.gpu, pytest.mark.xfail(strict=False, reason="first run on a GPU happens at round end")]
+pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("name", sorted(fc.CASES))
