@@ -166,120 +166,193 @@ k_project_rows(Cols in, int nk_in, const i64* w, u64 n, dbsp_proj proj, int iden
 }
 
 // ---------------- delta x trace probes -----------------------------------------
-// Per *distinct* delta key (delta rows are sorted, so a key's rows are one
-// segment [kstart[k], kstart[k+1])) and per trace batch: the range of trace rows
-// carrying that key — lower bound by bisection, upper bound by galloping (the
-// `seek_key` of cursor/mod.rs + advance.rs:25-72).  One search per key instead of
-// one per row; all spine batches in one launch.
-__global__ void k_probe_keys(Cols D, const u64* kstart, const u32* d_nkeys, BatchRefs tr, int nk, Flips f, u32* lo_out,
-                             u32* cnt_out, u32* ktot) {
-  const u64 gtid = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-  const u64 nkeys = (u64)*d_nkeys;   // the exact key count lives on the device; the grid is a fixed-size grid-stride loop
-  for (u64 k = gtid; k < nkeys; k += (u64)gridDim.x * blockDim.x) {
-    const u64 row = kstart[k];
-    u64 q[MAXL];
-    for (int l = 0; l < nk; l++) q[l] = D.c[l][row] ^ f.f[l];
-    u64 tot = 0;
-    for (int b = 0; b < tr.nb; b++) {
-      const Cols& T = tr.b[b].c;
-      const u64 nt = tr.b[b].n;
-      u64 lo = lower_bound_q(T, 0, nt, q, nk, f);
-      u64 hi = lo, step = 1;
-      while (hi + step <= nt && cmp_row_q(T, hi + step - 1, q, nk, f) == 0) { hi += step; step <<= 1; }
-      u64 top = hi + step <= nt ? hi + step : nt;
-      hi = upper_bound_q(T, hi, top, q, nk, f);
-      lo_out[k * tr.nb + b] = (u32)lo;
-      cnt_out[k * tr.nb + b] = (u32)(hi - lo);
-      tot += hi - lo;
+// One pass per chunk of (up to MAX_REFS) trace batches over ticketed tiles of PR_TILE sorted delta rows.  A segment
+// is a run of equal keys (first nk lanes) inside one tile: it starts at a key head or at the tile's first row, so a
+// key whose rows span tiles is searched once per tile and no tile waits on another except in the match-count
+// look-back.
+//  1. segments: ki[i] = first row of row i's segment; the tile's segment heads are listed in shared memory.
+//  2. windows: per batch, the rows [wl, wh) between the tile's first and last key, by 16-way half-warp searches
+//     whose pivots include both ends of the range, so a tile whose keys all lie outside a batch settles it in one
+//     round.  An empty window settles every segment of the tile for that batch without touching the batch again.
+//  3. ranges: per batch, every segment searches only inside the window — in shared memory when the window's key
+//     lanes fit PR_STAGE words, else in place: lower bound by bisection, upper bound by galloping (the `seek_key`
+//     of cursor/mod.rs + advance.rs:25-72).  lo/cnt[first_row * nb + b].
+//  4. counts: matches of a row = matches of its segment (saturated to u32, so a 64-bit total >= 2^32-1 still trips
+//     the host's guard), block scan + decoupled look-back: ex[i] = output slot of row i's first match, ex[nd] =
+//     total (32-bit, wraps on a rejected step); the last tile publishes the 64-bit total to the host mailbox.
+constexpr int PR_IPT = 4, PR_TILE = TB * PR_IPT, PR_STAGE = 2048;
+
+// bound of q in rows [lo,hi) of T — first row >= q, or > q when `upper` — searched by the 16 lanes of a half warp
+// (each lane one pivot per round).  Both halves of the warp must call it together; their ranges may differ.
+__device__ __forceinline__ u64 half_warp_bound(const Cols& T, u64 lo, u64 hi, const u64* q, int nk, const Flips& f,
+                                               bool upper) {
+  const int hl = threadIdx.x & 15, hs = threadIdx.x & 16;
+  while (true) {
+    const bool live = lo < hi;
+    if (!__any_sync(0xffffffffu, live)) break;
+    bool before = false;
+    if (live) {
+      const int c = cmp_row_q(T, lo + (u64)hl * (hi - lo - 1) / 15, q, nk, f);
+      before = upper ? c <= 0 : c < 0;
     }
-    ktot[k] = tot > 0xffffffffull ? 0xffffffffu : (u32)tot;   // saturate: the 64-bit total below then trips the guard
+    const int c = __popc((__ballot_sync(0xffffffffu, before) >> hs) & 0xffffu);   // pivots before the bound
+    if (live) {
+      const u64 span = hi - lo - 1;
+      if (c == 0) hi = lo;
+      else {
+        if (c < 16) hi = lo + (u64)c * span / 15;
+        lo = lo + (u64)(c - 1) * span / 15 + 1;
+      }
+    }
   }
+  return lo;
 }
 
-// Key segments of a sorted batch in one pass: a row is a head when it differs from its predecessor over the
-// first nk lanes.  Each thread owns SEG_IPT consecutive rows; block scan of the head counts + decoupled look-back
-// over the tiles give every head its key index: kstart[key] = row, ki[row] = key of the row, kstart[nkeys] = n
-// and *d_nkeys = nkeys (the key count never leaves the device).
-constexpr int SEG_IPT = 4, SEG_TILE = TB * SEG_IPT;
+// first staged row in [lo,hi) whose key is >= q (upper: > q); lane l of row j at s[l * ws + j]
+__device__ __forceinline__ u32 smem_bound(const u64* s, u32 ws, u32 lo, u32 hi, const u64* q, int nk, bool upper) {
+  while (lo < hi) {
+    const u32 mid = (lo + hi) >> 1;
+    int c = 0;
+    for (int l = 0; l < nk && c == 0; l++) {
+      const u64 a = s[l * ws + mid];
+      if (a != q[l]) c = a < q[l] ? -1 : 1;
+    }
+    if (upper ? c <= 0 : c < 0) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
 __global__ void __launch_bounds__(TB)
-k_key_segments(Cols C, u64 n, int nk, u32 ntiles, u32* ticket, u64* status, u64* kstart, u32* ki, u32* d_nkeys) {
-  __shared__ u32 s_tile, s_warp[TB / 32];
-  __shared__ u64 s_base;
+k_probe_ranges(Cols D, u64 nd, BatchRefs tr, int nk, Flips f, u32 ntiles, u32* ticket, u64* status, u32* ki, u32* lo_out,
+               u32* cnt_out, u32* ex, Mail mail) {
+  __shared__ u32 s_tile, s_wcnt[TB / 32], s_wl[MAX_REFS], s_wh[MAX_REFS];
+  __shared__ u64 s_wsum[TB / 32], s_base;
+  __shared__ u32 s_first[PR_TILE];   // first row (tile offset) of each segment
+  __shared__ u64 s_tot[PR_TILE];     // matches of each segment over the chunk's batches
+  __shared__ u64 s_stage[PR_STAGE];
   const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
   if (tid == 0) s_tile = atomicAdd(ticket, 1u);
   __syncthreads();
   const u32 t = s_tile;
-  const u64 i0 = (u64)t * SEG_TILE + (u64)tid * SEG_IPT;
+  const u64 t0 = (u64)t * PR_TILE;
+  const u64 tn = nd - t0 < (u64)PR_TILE ? nd - t0 : (u64)PR_TILE;   // rows of the tile
+  const int nb = tr.nb;
+
+  // 1. segments
+  const u32 r0 = (u32)tid * PR_IPT;
   unsigned heads = 0;
 #pragma unroll
-  for (int k = 0; k < SEG_IPT; k++) {
-    const u64 i = i0 + k;
-    if (i < n) {
-      bool head = i == 0;
+  for (int k = 0; k < PR_IPT; k++) {
+    const u64 i = t0 + r0 + k;
+    if (r0 + k < tn) {
+      bool head = r0 + k == 0;
       if (!head)
         for (int l = 0; l < nk; l++)
-          if (C.c[l][i] != C.c[l][i - 1]) { head = true; break; }
+          if (D.c[l][i] != D.c[l][i - 1]) { head = true; break; }
       heads |= (head ? 1u : 0u) << k;
     }
   }
-  const u32 cnt = __popc(heads);
-  u32 incl = cnt;
+  const u32 hc = __popc(heads);
+  u32 hincl = hc;
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) {
-    const u32 v = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += v;
+    const u32 v = __shfl_up_sync(0xffffffffu, hincl, o);
+    if (lane >= o) hincl += v;
   }
-  if (lane == 31) s_warp[wid] = incl;
-  __syncthreads();
-  u32 woff = 0, tile_total = 0;
-#pragma unroll
-  for (int k = 0; k < TB / 32; k++) {
-    const u32 v = s_warp[k];
-    if (k < wid) woff += v;
-    tile_total += v;
-  }
-  if (wid == 0) {
-    const u64 base = lb_exclusive_prefix(status, t, (u64)tile_total);
-    if (lane == 0) {
-      s_base = base;
-      if (t == ntiles - 1) {
-        *d_nkeys = (u32)(base + tile_total);
-        kstart[base + tile_total] = n;
+  if (lane == 31) s_wcnt[wid] = hincl;
+  // 2. windows: half warp h searches batch h / 2 (h even: lower bound of the first key, odd: upper bound of the
+  // last); both halves of a warp take the same number of rounds
+  {
+    const int h = tid >> 4;
+    const u64 qrow = (h & 1) ? t0 + tn - 1 : t0;
+    u64 q[MAXL];
+    for (int l = 0; l < nk; l++) q[l] = D.c[l][qrow] ^ f.f[l];
+    for (int s = h; s < 2 * nb; s += TB / 16) {
+      const int b = s >> 1;
+      const u64 bound = half_warp_bound(tr.b[b].c, 0, tr.b[b].n, q, nk, f, h & 1);
+      if ((tid & 15) == 0) {
+        if (h & 1) s_wh[b] = (u32)bound; else s_wl[b] = (u32)bound;
       }
     }
   }
   __syncthreads();
-  u32 run = (u32)s_base + woff + incl - cnt;   // heads before this thread's first row
+  u32 nseg = 0, woff = 0;
 #pragma unroll
-  for (int k = 0; k < SEG_IPT; k++) {
-    const u64 i = i0 + k;
-    if (i < n) {
-      if ((heads >> k) & 1) { kstart[run] = i; run++; }
-      ki[i] = run - 1;
+  for (int k = 0; k < TB / 32; k++) {
+    const u32 v = s_wcnt[k];
+    if (k < wid) woff += v;
+    nseg += v;
+  }
+  u32 seg[PR_IPT];   // segment of each of the thread's rows
+  {
+    u32 run = woff + hincl - hc;
+#pragma unroll
+    for (int k = 0; k < PR_IPT; k++) {
+      if ((heads >> k) & 1) { s_first[run] = r0 + k; run++; }
+      seg[k] = run - 1;
     }
   }
-}
-
-// matches of every delta row = matches of its key, and their exclusive running sum (the output slot of the row's
-// first match) in the same pass: ex[i] for i < nd, ex[nd] = total.  The total is carried in 64 bits through the
-// look-back (a skewed join can exceed 2^32 matches; the 32-bit ex[] wraps then, and the host rejects the step on
-// the exact total, which the last tile publishes to the host mailbox).
-__global__ void __launch_bounds__(TB)
-k_row_counts_scan(const u32* __restrict__ ki, const u32* __restrict__ ktot, u64 nd, u32 ntiles, u32* ticket, u64* status,
-                  u32* ex, Mail mail) {
-  __shared__ u32 s_tile;
-  __shared__ u64 s_warp[TB / 32];
-  __shared__ u64 s_base;
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  if (tid == 0) s_tile = atomicAdd(ticket, 1u);
   __syncthreads();
-  const u32 t = s_tile;
-  const u64 i0 = (u64)t * SEG_TILE + (u64)tid * SEG_IPT;
-  u32 c[SEG_IPT];
+
+  // 3. ranges: thread tid owns segments tid + j * TB for every batch
+  u64 tot[PR_IPT] = {};
+  for (int b = 0; b < nb; b++) {
+    const Cols& T = tr.b[b].c;
+    const u32 wl = s_wl[b], wh = s_wh[b], ws = wh - wl;
+    const bool staged = ws > 0 && (u64)ws * nk <= (u64)PR_STAGE;   // uniform over the CTA
+    if (staged) {
+      for (u32 x = tid; x < ws * (u32)nk; x += TB) {
+        const u32 l = x / ws, j = x - l * ws;
+        s_stage[x] = T.c[l][wl + j] ^ f.f[l];
+      }
+      __syncthreads();
+    }
+#pragma unroll
+    for (int j = 0; j < PR_IPT; j++) {
+      const u32 sg = (u32)tid + (u32)j * TB;
+      if (sg >= nseg) break;
+      const u64 row = t0 + s_first[sg];
+      u64 lo = wl, hi = wl;
+      if (ws > 0) {
+        u64 q[MAXL];
+        for (int l = 0; l < nk; l++) q[l] = D.c[l][row] ^ f.f[l];
+        if (staged) {
+          const u32 a = smem_bound(s_stage, ws, 0, ws, q, nk, false);
+          lo = wl + a;
+          hi = wl + smem_bound(s_stage, ws, a, ws, q, nk, true);
+        } else {
+          lo = lower_bound_q(T, wl, wh, q, nk, f);
+          u64 step = 1;
+          hi = lo;
+          while (hi + step <= wh && cmp_row_q(T, hi + step - 1, q, nk, f) == 0) { hi += step; step <<= 1; }
+          const u64 top = hi + step <= wh ? hi + step : wh;
+          hi = upper_bound_q(T, hi, top, q, nk, f);
+        }
+      }
+      lo_out[row * nb + b] = (u32)lo;
+      cnt_out[row * nb + b] = (u32)(hi - lo);
+      tot[j] += hi - lo;
+    }
+    if (staged) __syncthreads();
+  }
+#pragma unroll
+  for (int j = 0; j < PR_IPT; j++) {
+    const u32 sg = (u32)tid + (u32)j * TB;
+    if (sg < nseg) s_tot[sg] = tot[j];
+  }
+  __syncthreads();
+
+  // 4. counts and their exclusive prefix
+  u32 c[PR_IPT];
   u64 sum = 0;
 #pragma unroll
-  for (int k = 0; k < SEG_IPT; k++) {
-    c[k] = (i0 + k < nd) ? ktot[ki[i0 + k]] : 0u;
+  for (int k = 0; k < PR_IPT; k++) {
+    c[k] = 0;
+    if (r0 + k < tn) {
+      const u64 m = s_tot[seg[k]];
+      c[k] = m > 0xffffffffull ? 0xffffffffu : (u32)m;
+      ki[t0 + r0 + k] = (u32)t0 + s_first[seg[k]];
+    }
     sum += c[k];
   }
   u64 incl = sum;
@@ -288,13 +361,13 @@ k_row_counts_scan(const u32* __restrict__ ki, const u32* __restrict__ ktot, u64 
     const u64 v = __shfl_up_sync(0xffffffffu, incl, o);
     if (lane >= o) incl += v;
   }
-  if (lane == 31) s_warp[wid] = incl;
+  if (lane == 31) s_wsum[wid] = incl;
   __syncthreads();
-  u64 woff = 0, tile_total = 0;
+  u64 soff = 0, tile_total = 0;
 #pragma unroll
   for (int k = 0; k < TB / 32; k++) {
-    const u64 v = s_warp[k];
-    if (k < wid) woff += v;
+    const u64 v = s_wsum[k];
+    if (k < wid) soff += v;
     tile_total += v;
   }
   if (wid == 0) {
@@ -302,17 +375,17 @@ k_row_counts_scan(const u32* __restrict__ ki, const u32* __restrict__ ktot, u64 
     if (lane == 0) {
       s_base = base;
       if (t == ntiles - 1) {
-        const u64 tot = base + tile_total;
-        ex[nd] = (u32)tot;
-        mail_publish(mail, &tot, 1);
+        const u64 total = base + tile_total;
+        ex[nd] = (u32)total;
+        mail_publish(mail, &total, 1);
       }
     }
   }
   __syncthreads();
-  u64 run = s_base + woff + incl - sum;
+  u64 run = s_base + soff + incl - sum;
 #pragma unroll
-  for (int k = 0; k < SEG_IPT; k++) {
-    if (i0 + k < nd) ex[i0 + k] = (u32)run;
+  for (int k = 0; k < PR_IPT; k++) {
+    if (r0 + k < tn) ex[t0 + r0 + k] = (u32)run;
     run += c[k];
   }
 }
@@ -323,22 +396,25 @@ k_row_counts_scan(const u32* __restrict__ ki, const u32* __restrict__ ktot, u64 
 // needs no sort.  proj_mode 1: join_func(k, v1, v2) with filter
 // (join.rs:751-787), weight w1*w2, rejected rows keep their slot with weight 0;
 // proj_mode 0: copy the trace row (gather of a key group).
-// Load balancing: a CTA owns PF_TILE consecutive output slots whatever the fan-out of the keys behind them
-// (skew-proof).  Two threads bisect the scanned match counts for the delta rows of the tile's first and last
+// Load balancing: a CTA owns ipt * 256 consecutive output slots whatever the fan-out of the keys behind them
+// (skew-proof); the host picks ipt (1..PF_IPT) so that outputs of a few tens of thousands of slots still spread over
+// the SMs.  Two threads bisect the scanned match counts for the delta rows of the tile's first and last
 // slot; the counts in between are staged in shared memory, where every slot finds its delta row — one global
-// bisection per 1024 slots instead of one per slot.  Consecutive slots read consecutive trace rows and
-// the same / adjacent delta rows, and write consecutive output rows.
-constexpr int PF_TILE = 1024, PF_SMEM_ROWS = 3072;
+// bisection per tile instead of one per slot.  A slot's batch comes from its segment's nb counts, loaded side by
+// side (no load waits on another) and walked in registers.  Consecutive slots read consecutive trace rows and the same / adjacent delta rows,
+// and write consecutive output rows.
+constexpr int PF_IPT = 4, PF_SMEM_ROWS = 3072;
 __global__ void __launch_bounds__(256)
 k_probe_fill(Cols D, const i64* wD, u64 nd, BatchRefs tr, int nk, int nvD, int nvT, const u32* lo, const u32* cnt,
-             const u32* ki, const u32* exscan, u64 total, int proj_mode, int delta_is_left, dbsp_proj proj, MCols out,
-             i64* out_w) {
+             const u32* ki, const u32* exscan, u64 total, int ipt, int proj_mode, int delta_is_left, dbsp_proj proj,
+             MCols out, i64* out_w) {
   __shared__ u32 s_ex[PF_SMEM_ROWS + 1];
   __shared__ u64 s_rows[2];
   const int tid = threadIdx.x;
-  const u64 o0 = (u64)blockIdx.x * PF_TILE;
+  const u64 tile = (u64)ipt * 256;
+  const u64 o0 = (u64)blockIdx.x * tile;
   if (o0 >= total) return;
-  const u64 o1 = o0 + PF_TILE < total ? o0 + PF_TILE : total;
+  const u64 o1 = o0 + tile < total ? o0 + tile : total;
   if (tid < 2) {   // largest i with exscan[i] <= target
     const u64 target = tid == 0 ? o0 : o1 - 1;
     u64 a = 0, b = nd;
@@ -356,7 +432,7 @@ k_probe_fill(Cols D, const i64* wD, u64 nd, BatchRefs tr, int nk, int nvD, int n
     for (u64 k = tid; k <= nr; k += 256) s_ex[k] = exscan[row_lo + k];
   __syncthreads();
 #pragma unroll 1
-  for (int qq = 0; qq < PF_TILE / 256; qq++) {
+  for (int qq = 0; qq < ipt; qq++) {
     const u64 o = o0 + (u64)qq * 256 + tid;
     if (o >= o1) break;
     u64 i;
@@ -380,7 +456,13 @@ k_probe_fill(Cols D, const i64* wD, u64 nd, BatchRefs tr, int nk, int nvD, int n
     }
     const u64 kbase = (u64)ki[i] * tr.nb;
     int bb = 0;
-    while (bb < tr.nb - 1 && r >= cnt[kbase + bb]) { r -= cnt[kbase + bb]; bb++; }
+    u32 before = 0;   // matches in the batches before bb
+#pragma unroll 4
+    for (int b = 0; b < tr.nb - 1; b++) {   // load addresses do not depend on loaded counts: the loads overlap
+      const u32 c = cnt[kbase + b];
+      if (bb == b && r >= before + c) { before += c; bb = b + 1; }
+    }
+    r -= before;
     const Cols& T = tr.b[bb].c;
     const u64 t = (u64)lo[kbase + bb] + r;
     u64 row[MAXL];
@@ -893,44 +975,15 @@ int32_t project_and_consolidate(Ctx* ctx, const Cols& in, int nk_in, int n_in_la
   return consolidate_rows(ctx, os, t.cc(), t.w, m, &t.buf, out, d_m);
 }
 
-// Probe `delta` against every batch of `trace` and expand the matches.
-// proj == nullptr: gather the matching trace rows unchanged.
-// key segment starts of the first nk lanes: kstart[nkeys+1] (u64 row indices),
-// plus the key index of every row (u32[n]).
-static int32_t key_segments(Ctx* ctx, const Batch* b, int nk, BufP* kstart, BufP* ki, const u32** d_nkeys) {
-  // No read-back: the key count stays on the device; buffers and grids downstream are sized by the row count, an
-  // upper bound of it.  kstart: u64[n+1] (+ aux words behind it), ki: u32[n].
-  ROWS32(b->n, "key_segments");
-  const u64 n = b->n;
-  const u32 ntiles = (u32)((n + SEG_TILE - 1) / SEG_TILE);
-  // kstart[n+1] u64 | status[ntiles] u64 | ticket u32, nkeys u32
-  TRY(dev_alloc(ctx, (size_t)(n + 1 + ntiles + 1) * 8, kstart));
-  TRY(dev_alloc(ctx, (size_t)(n + 1) * 4, ki));
-  u64* ks = (u64*)(*kstart)->p;
-  u64* status = ks + (n + 1);
-  u32* ticket = (u32*)(status + ntiles);
-  u32* nkeys = ticket + 1;
-  CUDA_TRY(cudaMemsetAsync(status, 0, (size_t)(ntiles + 1) * 8, ctx->stream));
-  {
-    ProfScope ps(ctx, KID_PROBE_RANGES, n * (u64)nk * 8 + n * 12);
-    k_key_segments<<<ntiles, TB, 0, ctx->stream>>>(b->cols(), n, nk, ntiles, ticket, status, ks, (u32*)(*ki)->p, nkeys);
-  }
-  LAUNCH_COUNT(ctx);
-  *d_nkeys = nkeys;
-  return DBSP_OK;
-}
-
 // Probe `delta` against (up to MAX_REFS) batches of `trace` and expand the matches.
 // proj == nullptr: gather the matching trace rows unchanged.
 static int32_t probe_chunk(Ctx* ctx, const Batch* delta, int nk, Batch* const* tb, int nb, const dbsp_proj* proj,
-                           int delta_is_left, const dbsp_schema& out_schema, const u64* kstart, const u32* ki,
-                           const u32* d_nkeys, Batch** out) {
+                           int delta_is_left, const dbsp_schema& out_schema, Batch** out) {
   cudaStream_t st = ctx->stream;
   const u64 nd = delta->n;
   Flips f = delta->flips();
   BatchRefs refs;
   refs.nb = nb;
-  const u64 nkeys = nd;   // upper bound of the distinct keys (the exact count is *d_nkeys)
   u64 trace_rows = 0;
   ROWS32(nd, "join/gather delta");
   for (int b = 0; b < nb; b++) ROWS32(tb[b]->n, "join/gather trace batch");
@@ -940,34 +993,30 @@ static int32_t probe_chunk(Ctx* ctx, const Batch* delta, int nk, Batch* const* t
     refs.b[b].n = tb[b]->n;
     trace_rows += tb[b]->n;
   }
+  // lo, cnt: u32[nd * nb] (only the rows that start a segment are written) | ki: u32[nd]
   BufP kb, rb;
-  TRY(dev_alloc(ctx, (size_t)nkeys * nb * 4 * 2 + (size_t)nkeys * 4, &kb));
+  TRY(dev_alloc(ctx, (size_t)nd * nb * 4 * 2 + (size_t)nd * 4, &kb));
   u32* lo = (u32*)kb->p;
-  u32* cnt = lo + (size_t)nkeys * nb;
-  u32* ktot = cnt + (size_t)nkeys * nb;
+  u32* cnt = lo + (size_t)nd * nb;
+  u32* ki = cnt + (size_t)nd * nb;
   // ex[nd+1] u32 (padded to u64) | status[ntiles] u64 | ticket u64
-  const u32 ntiles = (u32)((nd + SEG_TILE - 1) / SEG_TILE);
+  const u32 ntiles = (u32)((nd + PR_TILE - 1) / PR_TILE);
   const size_t ex_u64 = (size_t)(nd + 2) / 2 + 1;
   TRY(dev_alloc(ctx, (ex_u64 + ntiles + 1) * 8, &rb));
   u32* ex = (u32*)rb->p;
   u64* status = (u64*)rb->p + ex_u64;
   u32* ticket = (u32*)(status + ntiles);
   CUDA_TRY(cudaMemsetAsync(status, 0, (size_t)(ntiles + 1) * 8, st));
-  {
-    // delta keys read once, ranges written once; every bisection step touches one
-    // trace key row (bounded by the trace's key bytes)
-    u64 lg = 1; while ((1ull << lg) < trace_rows / std::max(nb, 1) + 1) lg++;
-    u64 touched = std::min<u64>(nkeys * (u64)nb * 2 * lg, trace_rows) * (u64)std::max(nk, 1) * 8;
-    ProfScope ps(ctx, KID_PROBE_RANGES, nkeys * ((u64)nk * 8 + (u64)nb * 8 + 4) + touched);
-    const unsigned pg = (unsigned)std::min<u64>(blocks(nkeys), (u64)ctx->sm_count * 16);
-    k_probe_keys<<<pg, TB, 0, st>>>(delta->cols(), kstart, d_nkeys, refs, nk, f, lo, cnt, ktot);
-  }
   const Mail mail = mail_begin(ctx);
   {
-    ProfScope ps(ctx, KID_SCAN, nd * 16);
-    k_row_counts_scan<<<ntiles, TB, 0, st>>>(ki, ktot, nd, ntiles, ticket, status, ex, mail);
+    // delta key lanes read once; ki, lo, cnt and ex written once; every search step touches one trace key row
+    // (bounded by the trace's key bytes)
+    u64 lg = 1; while ((1ull << lg) < trace_rows / std::max(nb, 1) + 1) lg++;
+    const u64 touched = std::min<u64>(nd * (u64)nb * 2 * lg, trace_rows) * (u64)std::max(nk, 1) * 8;
+    ProfScope ps(ctx, KID_PROBE_RANGES, nd * ((u64)nk * 8 + (u64)nb * 8 + 8) + touched);
+    k_probe_ranges<<<ntiles, TB, 0, st>>>(delta->cols(), nd, refs, nk, f, ntiles, ticket, status, ki, lo, cnt, ex, mail);
   }
-  ctx->kernel_launches += 2;
+  LAUNCH_COUNT(ctx);
   u64 total;
   TRY(mail_finish(ctx, mail, &total, 1));
   if (total >= 0xffffffffull) {
@@ -984,8 +1033,13 @@ static int32_t probe_chunk(Ctx* ctx, const Batch* delta, int nk, Batch* const* t
     // matched trace rows read once, delta rows read once, output rows written once
     ProfScope ps(ctx, KID_PROBE_FILL, (u64)total * (u64)(tb[0]->nl() - nk + 1) * 8 + nd * (u64)(delta->nl() + 1) * 8 +
                                           (u64)total * (u64)(Lo + 1) * 8);
-    k_probe_fill<<<(unsigned)((total + PF_TILE - 1) / PF_TILE), 256, 0, st>>>(delta->cols(), delta->w, nd, refs, nk, delta->nl() - nk, tb[0]->nl() - nk, lo,
-                                               cnt, ki, ex, total, proj ? 1 : 0, delta_is_left, pj, t.c, t.w);
+    // slots per thread: as few as keep about two CTAs per SM busy, at most PF_IPT
+    const u64 per_pass = (u64)256 * 2 * ctx->sm_count;
+    const int ipt = (int)std::min<u64>(PF_IPT, std::max<u64>(1, (total + per_pass - 1) / per_pass));
+    const u64 tile = (u64)ipt * 256;
+    k_probe_fill<<<(unsigned)((total + tile - 1) / tile), 256, 0, st>>>(delta->cols(), delta->w, nd, refs, nk, delta->nl() - nk,
+                                                                        tb[0]->nl() - nk, lo, cnt, ki, ex, total, ipt,
+                                                                        proj ? 1 : 0, delta_is_left, pj, t.c, t.w);
   }
   LAUNCH_COUNT(ctx);
   // the Batcher of join.rs:845-858: usually sort-free (ordered slots)
@@ -998,15 +1052,11 @@ static int32_t probe_spine(Ctx* ctx, const Batch* delta, int nk, const Spine* tr
                            int delta_is_left, const dbsp_schema& out_schema, Batch** out) {
   const size_t nb = trace->batches.size();
   if (delta->n == 0 || nb == 0) { *out = batch_new_empty(ctx, out_schema); return DBSP_OK; }
-  BufP kstart, ki;
-  const u32* nkeys = nullptr;   // device count of the distinct delta keys
-  TRY(key_segments(ctx, delta, nk, &kstart, &ki, &nkeys));
   std::vector<Batch*> parts;
   for (size_t b0 = 0; b0 < nb; b0 += MAX_REFS) {
     int cnt = (int)std::min<size_t>(MAX_REFS, nb - b0);
     Batch* part = nullptr;
-    int32_t rc = probe_chunk(ctx, delta, nk, trace->batches.data() + b0, cnt, proj, delta_is_left, out_schema,
-                             (const u64*)kstart->p, (const u32*)ki->p, nkeys, &part);
+    int32_t rc = probe_chunk(ctx, delta, nk, trace->batches.data() + b0, cnt, proj, delta_is_left, out_schema, &part);
     if (rc) { for (Batch* p : parts) batch_unref(p); return rc; }
     parts.push_back(part);
   }
