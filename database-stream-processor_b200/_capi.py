@@ -50,6 +50,18 @@ class CProj(C.Structure):
     ]
 
 
+class CTableJob(C.Structure):
+    _fields_ = [
+        ("cols", C.c_void_p),
+        ("weights", C.c_void_p),
+        ("n", C.c_uint64),
+        ("upload", C.c_void_p),
+        ("proj", C.POINTER(CProj)),
+        ("n_cols", C.c_uint32),
+        ("on_device", C.c_int32),
+    ]
+
+
 class DbspError(RuntimeError):
     pass
 
@@ -129,19 +141,31 @@ _SIGS = {
     "gather": [_P, _P, C.c_int32, _PP],
     "allreduce_max_u64": [_P, _U64P],
 }
+# The grouped calls that run on the CUDA library's two execution lanes.  A library without them (the CPU oracle)
+# leaves them unbound and `zset.Backend` issues the same sequence of single calls instead.
+_GROUPED_SIGS = {
+    "batches_from_tables": [_P, C.c_uint32, C.POINTER(CTableJob), _PP],
+    "join_step": [_P, _P, _P, _P, _P, C.POINTER(CProj), _PP],
+}
 COMM_BLOB_BYTES = 128
 
 
 class CApi:
     """Thin, typed view of a shared library exporting the dbsp_b200.h ABI."""
 
-    def __init__(self, lib: C.CDLL, prefix: str):
+    def __init__(self, lib: C.CDLL, prefix: str, require_grouped: bool = False):
         self.lib = lib
         self.prefix = prefix
         for name, argtypes in _SIGS.items():
             fn = getattr(lib, prefix + name)  # AttributeError if a symbol is missing
             fn.argtypes = argtypes
             fn.restype = C.c_int32
+            setattr(self, "_" + name, fn)
+        for name, argtypes in _GROUPED_SIGS.items():
+            fn = getattr(lib, prefix + name) if require_grouped else getattr(lib, prefix + name, None)
+            if fn is not None:
+                fn.argtypes = argtypes
+                fn.restype = C.c_int32
             setattr(self, "_" + name, fn)
         self._last_error = getattr(lib, prefix + "last_error")
         self._last_error.restype = C.c_char_p
@@ -155,7 +179,7 @@ class CApi:
 
     @staticmethod
     def symbols(prefix: str = "dbsp_"):
-        return [prefix + n for n in list(_SIGS) + ["last_error", "ctx_stream", "proj_table_mask"]]
+        return [prefix + n for n in list(_SIGS) + list(_GROUPED_SIGS) + ["last_error", "ctx_stream", "proj_table_mask"]]
 
     def check(self, rc: int, what: str):
         if rc != OK:

@@ -38,7 +38,9 @@ class FoldSum:  # Fold summing distinct values (aggregate/mod.rs:918-929)
 
 
 class Node:
-    def __init__(self, circuit: "RootCircuit", inputs: Sequence["Node"], fn: Callable, name: str):
+    table_proj = None   # set on the flat_map_index of a raw table, which `RootCircuit.step` evaluates in groups
+
+    def __init__(self, circuit: "RootCircuit", inputs: Sequence["Node"], fn: Callable | None, name: str):
         self.circuit, self.inputs, self.fn, self.name = circuit, list(inputs), fn, name
         self.value = None
         circuit.nodes.append(self)
@@ -130,8 +132,26 @@ class RootCircuit:
         return Stream(self, node, schema)
 
     def step(self):
+        done = set()
         for n in self.nodes:
-            n.eval()
+            if id(n) in done:
+                continue
+            if n.table_proj is not None:
+                # every table projection whose table is already evaluated, in one call: the library ingests the
+                # tables side by side on its two execution lanes
+                group = [m for m in self.nodes if m.table_proj is not None and id(m) not in done and id(m.inputs[0]) in done]
+                self._eval_tables(group)
+                done.update(id(m) for m in group)
+            else:
+                n.eval()
+                done.add(id(n))
+
+    def _eval_tables(self, group):
+        live = [(m, m.table_proj) for m in group if m.inputs[0].value is not None]
+        outs = self.be.batches_from_tables([(m.inputs[0].value, p) for m, p in live]) if live else []
+        got = {id(m): b for (m, _), b in zip(live, outs)}
+        for m in group:
+            m.value = got[id(m)] if id(m) in got else self.be.batch_empty(m.table_proj.schema)
 
     @property
     def workers(self):
@@ -152,19 +172,13 @@ class TableStream:
 
     def flat_map_index(self, proj: Proj) -> "Stream":
         """flat_map_index on the event stream (filter_map.rs:143-152,700-724):
-        filter + project + from_tuples, straight from the raw columns."""
-        be = self.circuit.be
+        filter + project + from_tuples, straight from the raw columns
+        (evaluated by `RootCircuit.step` together with the circuit's other
+        table projections)."""
         self.projs.append(proj)
-
-        def fn(t):
-            if t is None:
-                return be.batch_empty(proj.schema)
-            kind, cols, w, n = t
-            if kind == "upload":
-                return be.batch_from_upload(cols, proj)
-            return be.batch_from_table(cols, proj, weights=w, n=n, on_device=(kind == "dev"))
-
-        return Stream(self.circuit, Node(self.circuit, [self.node], fn, "flat_map_index"), proj.schema)
+        node = Node(self.circuit, [self.node], None, "flat_map_index")
+        node.table_proj = proj
+        return Stream(self.circuit, node, proj.schema)
 
 
 class Stream:
@@ -295,11 +309,9 @@ class Stream:
         lt, rt = Spine(be, left.schema), Spine(be, right.schema)
 
         def fn(dl: Batch, dr: Batch):
-            rt.insert(dr)                                            # right.trace()
-            o1 = be.join_delta_trace(dl, rt, proj, delta_is_left=True)
-            o2 = be.join_delta_trace(dr, lt, proj, delta_is_left=False)  # vs delayed left trace
-            lt.insert(dl)                                            # left.trace()
-            return be.merge(o1, o2)                                  # left.plus(&right)
+            # rt.insert(dr) (right.trace()); o1 = dl |x| rt; o2 = dr |x| z^-1(lt); lt.insert(dl) (left.trace());
+            # o1 + o2 (left.plus(&right)) — the halves run side by side in the library
+            return be.join_step(dl, dr, lt, rt, proj)
 
         return left._binary(right, fn, "join", proj.schema)
 

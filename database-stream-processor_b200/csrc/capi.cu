@@ -1,6 +1,7 @@
 // capi.cu — the extern "C" boundary declared in include/dbsp_b200.h, plus the
 // host-side Spine (trace) logic.  No CPU compute path lives here: every
 // data-touching call launches kernels from consolidate.cu / merge.cu / ops.cu.
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 
@@ -44,13 +45,13 @@ static int32_t stage_columns(Ctx* ctx, const u64* const* cols, int ncols, const 
   u64* base = (u64*)(*hold)->p;
   for (int l = 0; l < ncols; l++) {
     if (!((col_mask >> l) & 1)) continue;   // column never read by the closure: not copied
-    CUDA_TRY(cudaMemcpyAsync(base + (size_t)l * cap, cols[l], n * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(base + (size_t)l * cap, cols[l], n * 8, cudaMemcpyHostToDevice, lane(ctx).stream));
     dc->c[l] = base + (size_t)l * cap;
     ctx->h2d_bytes += n * 8;
   }
   if (w) {
     i64* p = (i64*)(base + (size_t)ncols * cap);
-    CUDA_TRY(cudaMemcpyAsync(p, w, n * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(p, w, n * 8, cudaMemcpyHostToDevice, lane(ctx).stream));
     ctx->h2d_bytes += n * 8;
     *dw = p;
   }
@@ -349,21 +350,28 @@ int32_t dbsp_ctx_create(int32_t device, dbsp_ctx** out) {
   CUDA_TRY(cudaSetDevice(device));
   dbsp_ctx* c = new dbsp_ctx();
   c->device = device;
-  CUDA_TRY(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
   CUDA_TRY(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
   CUDA_TRY(cudaStreamCreateWithFlags(&c->read_stream, cudaStreamNonBlocking));
   CUDA_TRY(cudaMallocHost(&c->h_scratch, 256 * 8));
   {
+    // one mailbox slot (320 words) and 256 scratch words per lane
     void* hm = nullptr;
-    CUDA_TRY(cudaHostAlloc(&hm, 320 * 8, cudaHostAllocMapped));
-    memset(hm, 0, 320 * 8);
-    c->h_mail = (volatile u64*)hm;
+    CUDA_TRY(cudaHostAlloc(&hm, N_LANES * 320 * 8, cudaHostAllocMapped));
+    memset(hm, 0, N_LANES * 320 * 8);
     void* dm = nullptr;
     CUDA_TRY(cudaHostGetDevicePointer(&dm, hm, 0));
-    c->d_mail = (u64*)dm;
+    u64* ds = nullptr;
+    CUDA_TRY(cudaMalloc(&ds, N_LANES * 256 * 8));
+    CUDA_TRY(cudaMemset(ds, 0, N_LANES * 256 * 8));
+    for (int i = 0; i < N_LANES; i++) {
+      Lane& l = c->lanes[i];
+      CUDA_TRY(cudaStreamCreateWithFlags(&l.stream, cudaStreamNonBlocking));
+      CUDA_TRY(cudaEventCreateWithFlags(&l.ev, cudaEventDisableTiming));
+      l.h_mail = (volatile u64*)hm + i * 320;
+      l.d_mail = (u64*)dm + i * 320;
+      l.d_scratch = ds + i * 256;
+    }
   }
-  CUDA_TRY(cudaMalloc(&c->d_scratch, 256 * 8));
-  CUDA_TRY(cudaMemset(c->d_scratch, 0, 256 * 8));
   cudaDeviceProp prop;
   CUDA_TRY(cudaGetDeviceProperties(&prop, device));
   c->sm_count = prop.multiProcessorCount;
@@ -388,62 +396,71 @@ int32_t dbsp_ctx_destroy(dbsp_ctx* c) {
   if (!c) return DBSP_OK;
   print_host_stats(c);
   cudaSetDevice(c->device);
-  cudaStreamSynchronize(c->stream);
+  lanes_shutdown(c);
+  for (Lane& l : c->lanes) cudaStreamSynchronize(l.stream);
   comm_free(c);
   cudaFreeHost(c->h_scratch);
-  cudaFreeHost((void*)c->h_mail);
-  cudaFree(c->d_scratch);
+  cudaFreeHost((void*)c->lanes[0].h_mail);
+  cudaFree(c->lanes[0].d_scratch);
   pool_release_all(c);
-  for (auto& r : c->prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
-  for (auto& e : c->ev_pool) cudaEventDestroy(e);
-  c->prof.clear();
-  c->ev_pool.clear();
-  cudaStreamDestroy(c->stream);
+  for (Lane& l : c->lanes) {
+    for (auto& r : l.prof) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
+    for (auto& e : l.ev_pool) cudaEventDestroy(e);
+    l.prof.clear();
+    l.ev_pool.clear();
+    cudaEventDestroy(l.ev);
+    cudaStreamDestroy(l.stream);
+    l.stream = nullptr;
+  }
   cudaStreamDestroy(c->copy_stream);
   cudaStreamDestroy(c->read_stream);
-  c->stream = nullptr;
   c->destroyed = true;
   if (c->live_bufs.load() == 0) delete c;   // else the last DevBuf deletes it
   return DBSP_OK;
 }
 int32_t dbsp_ctx_sync(dbsp_ctx* c) { ENTER(c);
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->lanes[0].stream));   // lane 0 waits for lane 1 at every join
   return DBSP_OK;
 }
 int32_t dbsp_ctx_stats(dbsp_ctx* c, uint64_t* k, uint64_t* h2d, uint64_t* d2h, int32_t reset) { ENTER(c);
   if (k) *k = c->kernel_launches;
   if (h2d) *h2d = c->h2d_bytes;
   if (d2h) *d2h = c->d2h_bytes;
-  if (reset) c->kernel_launches = c->h2d_bytes = c->d2h_bytes = 0;
+  if (reset) { c->kernel_launches = 0; c->h2d_bytes = 0; c->d2h_bytes = 0; }
   return DBSP_OK;
 }
 int32_t dbsp_ctx_sync_stats(dbsp_ctx* c, uint64_t* n_waits, double* wait_us, int32_t reset) {
-  if (n_waits) *n_waits = c->n_sync;
-  if (wait_us) *wait_us = c->t_sync_us;
-  if (reset) { c->n_sync = 0; c->t_sync_us = 0; }
+  // both lanes: waits on lane 1 overlap lane 0's work, so wait_us may exceed the wall time it covers
+  if (n_waits) *n_waits = c->lanes[0].n_sync + c->lanes[1].n_sync;
+  if (wait_us) *wait_us = c->lanes[0].t_sync_us + c->lanes[1].t_sync_us;
+  if (reset) for (Lane& l : c->lanes) { l.n_sync = 0; l.t_sync_us = 0; }
   return DBSP_OK;
 }
-void* dbsp_ctx_stream(dbsp_ctx* c) { return (void*)c->stream; }
+void* dbsp_ctx_stream(dbsp_ctx* c) { return (void*)c->lanes[0].stream; }
 
 int32_t dbsp_ctx_profile(dbsp_ctx* c, int32_t enable) { ENTER(c);
   if (enable == 2) { c->prof_on = false; return DBSP_OK; }   // pause: keep what was collected, record nothing more
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
-  for (auto& r : c->prof) { c->ev_pool.push_back(r.a); c->ev_pool.push_back(r.b); }
-  c->prof.clear();
+  CUDA_TRY(cudaStreamSynchronize(c->lanes[0].stream));
+  for (Lane& l : c->lanes) {
+    for (auto& r : l.prof) { l.ev_pool.push_back(r.a); l.ev_pool.push_back(r.b); }
+    l.prof.clear();
+  }
   c->prof_on = enable != 0;
   return DBSP_OK;
 }
 int32_t dbsp_ctx_profile_read(dbsp_ctx* c, int32_t id, char* name32, uint64_t* launches, double* ms, uint64_t* bytes) { ENTER(c);
   if (id < 0 || id >= KID_COUNT) return DBSP_ERR_INVALID;
-  CUDA_TRY(cudaStreamSynchronize(c->stream));
+  CUDA_TRY(cudaStreamSynchronize(c->lanes[0].stream));
   u64 n = 0, b = 0;
   double t = 0;
-  for (auto& r : c->prof) {
-    if (r.id != id) continue;
-    float e = 0;
-    if (cudaEventElapsedTime(&e, r.a, r.b) == cudaSuccess) t += e;
-    n++;
-    b += r.bytes;
+  for (Lane& l : c->lanes) {
+    for (auto& r : l.prof) {
+      if (r.id != id) continue;
+      float e = 0;
+      if (cudaEventElapsedTime(&e, r.a, r.b) == cudaSuccess) t += e;
+      n++;
+      b += r.bytes;
+    }
   }
   if (name32) { strncpy(name32, kernel_name(id), 31); name32[31] = 0; }
   if (launches) *launches = n;
@@ -466,19 +483,6 @@ int32_t dbsp_batch_from_tuples(dbsp_ctx* ctx, const dbsp_schema* s, const uint64
   return DBSP_OK;
 }
 
-int32_t dbsp_batch_from_table(dbsp_ctx* ctx, const uint64_t* const* cols, uint32_t n_cols, const int64_t* w, uint64_t n,
-                              int32_t on_device, const dbsp_proj* proj, dbsp_batch** out) { ENTER(ctx);
-  CHECK_ARG(n_cols >= 1 && n_cols <= MAXL, "table must have 1..8 columns");
-  BufP hold;
-  Cols dc;
-  const i64* dw;
-  TRY(stage_columns(ctx, cols, (int)n_cols, w, n, on_device, &hold, &dc, &dw, proj_used_mask(*proj, 0)));
-  Batch* b = nullptr;
-  TRY(project_and_consolidate(ctx, dc, 0, (int)n_cols, dw, n, *proj, &b));
-  *out = H(b);
-  return DBSP_OK;
-}
-
 struct dbsp_upload {
   Ctx* ctx;
   BufP buf;
@@ -488,6 +492,59 @@ struct dbsp_upload {
   int n_cols;
   cudaEvent_t done;
 };
+
+// flat_map_index of one raw table on the calling thread's lane
+static int32_t table_to_batch(Ctx* ctx, const dbsp_table_job& j, Batch** out) {
+  CHECK_ARG(j.proj != nullptr, "table: projection is NULL");
+  if (j.upload) {
+    CUDA_TRY(cudaStreamWaitEvent(lane(ctx).stream, j.upload->done, 0));   // the lane waits for the copy
+    return project_and_consolidate(ctx, j.upload->dc, 0, j.upload->n_cols, j.upload->dw, j.upload->n, *j.proj, out);
+  }
+  CHECK_ARG(j.n_cols >= 1 && j.n_cols <= MAXL, "table must have 1..8 columns");
+  BufP hold;
+  Cols dc;
+  const i64* dw;
+  TRY(stage_columns(ctx, j.cols, (int)j.n_cols, j.weights, j.n, j.on_device, &hold, &dc, &dw, proj_used_mask(*j.proj, 0)));
+  return project_and_consolidate(ctx, dc, 0, (int)j.n_cols, dw, j.n, *j.proj, out);
+}
+
+int32_t dbsp_batch_from_table(dbsp_ctx* ctx, const uint64_t* const* cols, uint32_t n_cols, const int64_t* w, uint64_t n,
+                              int32_t on_device, const dbsp_proj* proj, dbsp_batch** out) { ENTER(ctx);
+  dbsp_table_job j = {cols, w, n, nullptr, proj, n_cols, on_device};
+  Batch* b = nullptr;
+  TRY(table_to_batch(ctx, j, &b));
+  *out = H(b);
+  return DBSP_OK;
+}
+
+int32_t dbsp_batches_from_tables(dbsp_ctx* ctx, uint32_t k, const dbsp_table_job* jobs, dbsp_batch** outs) { ENTER(ctx);
+  CHECK_ARG(k == 0 || (jobs && outs), "batches_from_tables: jobs / outs is NULL");
+  // Largest table first, each onto the lane with fewer rows so far: lane 0 (this thread) starts on the largest one
+  // while the worker picks up its share.
+  std::vector<uint32_t> order(k);
+  for (uint32_t i = 0; i < k; i++) order[i] = i;
+  auto rows = [&](uint32_t i) { return jobs[i].upload ? jobs[i].upload->n : jobs[i].n; };
+  std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return rows(a) > rows(b); });
+  std::vector<uint32_t> on[N_LANES];
+  u64 load[N_LANES] = {0, 0};
+  for (uint32_t i : order) {
+    const int l = load[1] < load[0] ? 1 : 0;
+    on[l].push_back(i);
+    load[l] += rows(i);
+  }
+  std::vector<Batch*> o(k, nullptr);
+  auto run = [&](const std::vector<uint32_t>& js) -> int32_t {
+    for (uint32_t i : js) TRY(table_to_batch(ctx, jobs[i], &o[i]));
+    return DBSP_OK;
+  };
+  const int32_t rc = on[1].empty() ? run(on[0]) : run_forked(ctx, [&] { return run(on[0]); }, [&] { return run(on[1]); });
+  if (rc != DBSP_OK) {
+    for (Batch* b : o) batch_unref(b);
+    return rc;
+  }
+  for (uint32_t i = 0; i < k; i++) outs[i] = H(o[i]);
+  return DBSP_OK;
+}
 
 uint32_t dbsp_proj_table_mask(const dbsp_proj* proj) { return proj_used_mask(*proj, 0); }
 
@@ -507,7 +564,7 @@ int32_t dbsp_upload_begin(dbsp_ctx* ctx, const uint64_t* const* cols, uint32_t n
     // the block may have been used by work still queued on the compute stream
     cudaEvent_t ev;
     CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-    CUDA_TRY(cudaEventRecord(ev, ctx->stream));
+    CUDA_TRY(cudaEventRecord(ev, lane(ctx).stream));
     CUDA_TRY(cudaStreamWaitEvent(ctx->copy_stream, ev, 0));
     CUDA_TRY(cudaEventDestroy(ev));
     u64* base = (u64*)u->buf->p;
@@ -530,9 +587,9 @@ int32_t dbsp_upload_begin(dbsp_ctx* ctx, const uint64_t* const* cols, uint32_t n
 }
 
 int32_t dbsp_batch_from_upload(dbsp_ctx* ctx, dbsp_upload* u, const dbsp_proj* proj, dbsp_batch** out) { ENTER(ctx);
-  CUDA_TRY(cudaStreamWaitEvent(ctx->stream, u->done, 0));   // compute stream waits for the copy
+  dbsp_table_job j = {nullptr, nullptr, 0, u, proj, 0, 0};
   Batch* b = nullptr;
-  TRY(project_and_consolidate(ctx, u->dc, 0, u->n_cols, u->dw, u->n, *proj, &b));
+  TRY(table_to_batch(ctx, j, &b));
   *out = H(b);
   return DBSP_OK;
 }
@@ -556,9 +613,9 @@ int32_t dbsp_batch_from_sorted(dbsp_ctx* ctx, const dbsp_schema* s, const uint64
   i64* ow;
   TRY(batch_alloc(ctx, *s, n, &b, &oc, &ow));
   cudaMemcpyKind kind = on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-  for (int l = 0; l < L; l++) CUDA_TRY(cudaMemcpyAsync(oc.c[l], cols[l], n * 8, kind, ctx->stream));
-  CUDA_TRY(cudaMemcpyAsync(ow, w, n * 8, kind, ctx->stream));
-  if (!on_device) { ctx->h2d_bytes += n * 8 * (L + 1); CUDA_TRY(cudaStreamSynchronize(ctx->stream)); }
+  for (int l = 0; l < L; l++) CUDA_TRY(cudaMemcpyAsync(oc.c[l], cols[l], n * 8, kind, lane(ctx).stream));
+  CUDA_TRY(cudaMemcpyAsync(ow, w, n * 8, kind, lane(ctx).stream));
+  if (!on_device) { ctx->h2d_bytes += n * 8 * (L + 1); CUDA_TRY(cudaStreamSynchronize(lane(ctx).stream)); }
   *out = H(b);
   return DBSP_OK;
 }
@@ -766,7 +823,7 @@ int32_t dbsp_batch_schema(const dbsp_batch* b, dbsp_schema* out) { *out = B(b)->
 int32_t dbsp_batch_download_csr(dbsp_ctx* ctx, const dbsp_batch* bb, uint64_t* const* keys, uint64_t* offs,
                                 uint64_t* const* vals, int64_t* diffs) { ENTER(ctx);
   Batch* b = B(bb);
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = lane(ctx).stream;
   int nk = b->s.n_key_lanes, nv = b->s.n_val_lanes;
   if (b->n == 0) { if (offs && nv) offs[0] = 0; return DBSP_OK; }
   if (nv == 0) {
@@ -810,7 +867,7 @@ int32_t dbsp_batch_download_begin(dbsp_ctx* ctx, const dbsp_batch* bb, uint64_t*
       // the read stream picks the batch up once the kernels that produce it have run
       cudaEvent_t ev;
       CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-      cudaError_t e1 = cudaEventRecord(ev, ctx->stream);
+      cudaError_t e1 = cudaEventRecord(ev, lane(ctx).stream);
       cudaError_t e2 = cudaStreamWaitEvent(ctx->read_stream, ev, 0);
       cudaEventDestroy(ev);
       CUDA_TRY(e1);
@@ -864,9 +921,9 @@ int32_t dbsp_batch_last_key(dbsp_ctx* ctx, const dbsp_batch* b, uint64_t* key, i
   *valid = x->n > 0;
   if (!x->n) return DBSP_OK;
   for (int l = 0; l < x->s.n_key_lanes; l++) {
-    CUDA_TRY(cudaMemcpyAsync(ctx->h_scratch + l, x->col[l] + (x->n - 1), 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(ctx->h_scratch + l, x->col[l] + (x->n - 1), 8, cudaMemcpyDeviceToHost, lane(ctx).stream));
   }
-  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  CUDA_TRY(cudaStreamSynchronize(lane(ctx).stream));
   for (int l = 0; l < x->s.n_key_lanes; l++) key[l] = ctx->h_scratch[l];
   ctx->d2h_bytes += 8 * x->s.n_key_lanes;
   return DBSP_OK;
@@ -972,8 +1029,8 @@ static int32_t save_batch(Ctx* ctx, FILE* f, const Batch* b, std::vector<u64>& s
     const void* src = l < L ? (const void*)b->col[l] : (const void*)b->w;
     for (u64 off = 0; off < n; off += stage.size()) {
       const u64 m = std::min<u64>(stage.size(), n - off);
-      CUDA_TRY(cudaMemcpyAsync(stage.data(), (const u64*)src + off, m * 8, cudaMemcpyDeviceToHost, ctx->stream));
-      CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+      CUDA_TRY(cudaMemcpyAsync(stage.data(), (const u64*)src + off, m * 8, cudaMemcpyDeviceToHost, lane(ctx).stream));
+      CUDA_TRY(cudaStreamSynchronize(lane(ctx).stream));
       ctx->d2h_bytes += m * 8;
       if (!fwrite_all(f, stage.data(), m * 8)) { set_error("spine_save: write failed"); return DBSP_ERR_INVALID; }
     }
@@ -996,8 +1053,8 @@ static int32_t load_batch(Ctx* ctx, FILE* f, const dbsp_schema& sc, Batch** out,
     for (u64 off = 0; off < n; off += stage.size()) {
       const u64 m = std::min<u64>(stage.size(), n - off);
       if (!fread_all(f, stage.data(), m * 8)) { batch_unref(b); set_error("spine_load: truncated file"); return DBSP_ERR_INVALID; }
-      cudaError_t e = cudaMemcpyAsync(dst + off, stage.data(), m * 8, cudaMemcpyHostToDevice, ctx->stream);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+      cudaError_t e = cudaMemcpyAsync(dst + off, stage.data(), m * 8, cudaMemcpyHostToDevice, lane(ctx).stream);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(lane(ctx).stream);
       if (e != cudaSuccess) { batch_unref(b); set_error(cudaGetErrorString(e)); return DBSP_ERR_CUDA; }
       ctx->h2d_bytes += m * 8;
     }
@@ -1071,6 +1128,34 @@ int32_t dbsp_spine_load(dbsp_ctx* ctx, const char* path, dbsp_spine** out) { ENT
 
 int32_t dbsp_join_delta_trace(dbsp_ctx* ctx, const dbsp_batch* d, const dbsp_spine* t, const dbsp_proj* p, int32_t dl,
                               dbsp_batch** out) { ENTER(ctx); OUT1(op_join_delta_trace(ctx, B(d), t, p, dl, &o__)) }
+// The join operator (join.rs:180-292) over one step: lane 0 inserts δright into the right trace and joins δleft
+// with it; lane 1 joins δright with the left trace as it was before this step (z^-1) and then inserts δleft.  The
+// halves touch different traces, so each trace sees the same operations as in the sequential order.
+int32_t dbsp_join_step(dbsp_ctx* ctx, const dbsp_batch* dl, const dbsp_batch* dr, dbsp_spine* lt, dbsp_spine* rt,
+                       const dbsp_proj* p, dbsp_batch** out) { ENTER(ctx);
+  CHECK_ARG(dl && dr && lt && rt && p && out, "join_step: NULL argument");
+  CHECK_ARG(lt != rt, "join_step: the left and right traces must differ");
+  CHECK_ARG(memcmp(&lt->s, &B(dl)->s, sizeof(dbsp_schema)) == 0, "join_step: left delta / trace schema mismatch");
+  CHECK_ARG(memcmp(&rt->s, &B(dr)->s, sizeof(dbsp_schema)) == 0, "join_step: right delta / trace schema mismatch");
+  Batch *o1 = nullptr, *o2 = nullptr;
+  int32_t rc = run_forked(
+      ctx,
+      [&]() -> int32_t {
+        TRY(spine_insert(ctx, rt, B(dr)));
+        return op_join_delta_trace(ctx, B(dl), rt, p, 1, &o1);
+      },
+      [&]() -> int32_t {
+        TRY(op_join_delta_trace(ctx, B(dr), lt, p, 0, &o2));
+        return spine_insert(ctx, lt, B(dl));
+      });
+  Batch* o = nullptr;
+  if (rc == DBSP_OK) rc = merge_batches(ctx, o1, o2, &o);
+  batch_unref(o1);
+  batch_unref(o2);
+  if (rc != DBSP_OK) return rc;
+  *out = H(o);
+  return DBSP_OK;
+}
 int32_t dbsp_join_batches(dbsp_ctx* ctx, const dbsp_batch* l, const dbsp_batch* r, const dbsp_proj* p, dbsp_batch** out) { ENTER(ctx);
   OUT1(op_join_batches(ctx, B(l), B(r), p, &o__)) }
 int32_t dbsp_semijoin(dbsp_ctx* ctx, const dbsp_batch* pairs, const dbsp_batch* keys, dbsp_batch** out) { ENTER(ctx);
@@ -1103,7 +1188,7 @@ int32_t dbsp_comm_connect(dbsp_ctx* ctx, const uint8_t* blobs) { ENTER(ctx);
   return comm_connect(ctx, blobs);
 }
 int32_t dbsp_comm_destroy(dbsp_ctx* ctx) { ENTER(ctx);
-  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+  CUDA_TRY(cudaStreamSynchronize(lane(ctx).stream));
   comm_free(ctx);
   return DBSP_OK;
 }

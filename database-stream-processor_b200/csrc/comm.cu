@@ -435,7 +435,7 @@ static int32_t merge_views(Ctx* ctx, std::vector<Batch*>& parts, const dbsp_sche
     for (int l = 0; l < MAXL; l++) f.f[l] = (l < L && s.lane_types[l] == DBSP_I64) ? 0x8000000000000000ull : 0ull;
     {
       ProfScope ps(ctx, KID_SHARD, total * (u64)(L + 1) * 8 * 2);
-      k_pway_rank<<<(unsigned)((total + 255) / 256), 256, 0, ctx->stream>>>(sl, L, f, total, cap, (u64*)buf->p);
+      k_pway_rank<<<(unsigned)((total + 255) / 256), 256, 0, ctx->lanes[0].stream>>>(sl, L, f, total, cap, (u64*)buf->p);
     }
     LAUNCH_COUNT(ctx);
     for (Batch* b : live) batch_unref(b);
@@ -467,8 +467,8 @@ static int32_t merge_views(Ctx* ctx, std::vector<Batch*>& parts, const dbsp_sche
     rc = batch_alloc(ctx, s, r->n, &o, &oc, &ow);
     if (rc) { batch_unref(r); return rc; }
     const int L = s.n_key_lanes + s.n_val_lanes;
-    for (int l = 0; l < L; l++) cudaMemcpyAsync(oc.c[l], r->col[l], r->n * 8, cudaMemcpyDeviceToDevice, ctx->stream);
-    cudaMemcpyAsync(ow, r->w, r->n * 8, cudaMemcpyDeviceToDevice, ctx->stream);
+    for (int l = 0; l < L; l++) cudaMemcpyAsync(oc.c[l], r->col[l], r->n * 8, cudaMemcpyDeviceToDevice, ctx->lanes[0].stream);
+    cudaMemcpyAsync(ow, r->w, r->n * 8, cudaMemcpyDeviceToDevice, ctx->lanes[0].stream);
     batch_unref(r);
     r = o;
   }
@@ -479,13 +479,15 @@ static int32_t merge_views(Ctx* ctx, std::vector<Batch*>& parts, const dbsp_sche
 // One exchange round for `ns` (1 or 2) streams.  fixed_dest >= 0: every row goes to that rank (gather).
 int32_t comm_exchange(Ctx* ctx, const Batch* const* in, int ns, int fixed_dest, Batch** out) {
   Comm* c = ctx->comm;
+  // the exchange runs on lane 0 and its peers expect one round at a time
+  if (t_lane != 0 || ctx->fork_open) { set_error("exchange: called inside a fork of the execution lanes"); return DBSP_ERR_INVALID; }
   if (!c || c->world == 1) {
     for (int i = 0; i < ns; i++) { batch_ref((Batch*)in[i]); out[i] = (Batch*)in[i]; }
     return DBSP_OK;
   }
   if (!c->connected) { set_error("exchange: dbsp_comm_connect has not been called"); return DBSP_ERR_INVALID; }
   if (ns < 1 || ns > MAX_STREAMS) { set_error("exchange: 1 or 2 streams per round"); return DBSP_ERR_INVALID; }
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = ctx->lanes[0].stream;
   const u32 P = (u32)c->world;
   const u64 seq = ++c->seq;
   const int par = (int)(seq & 1);
@@ -542,14 +544,14 @@ int32_t comm_exchange(Ctx* ctx, const Batch* const* in, int ns, int fixed_dest, 
     ctx->kernel_launches += 3;
   }
   k_comm_signal<<<1, MAXP, 0, st>>>(sg, P, ns, totals[0], ns > 1 ? totals[1] : nullptr, err, seq);
-  const u64 mseq = ++ctx->mail_seq;
+  const u64 mseq = ++ctx->lanes[0].mail_seq;
   k_comm_wait<<<1, 32, 0, st>>>(((Ctrl*)c->region)->flags[par], P, seq, totals[0], ns > 1 ? totals[1] : nullptr,
-                                                   (volatile u64*)ctx->d_mail, mseq, comm_timeout_ns());
+                                                   (volatile u64*)ctx->lanes[0].d_mail, mseq, comm_timeout_ns());
   ctx->kernel_launches += 2;
   TRY(mail_wait(ctx, mseq));
-  ctx->n_sync++;
+  ctx->lanes[0].n_sync++;
   u64 hc[4 * MAXP + 1];
-  for (u32 k = 0; k < 4 * P + 1; k++) hc[k] = ctx->h_mail[8 + k];
+  for (u32 k = 0; k < 4 * P + 1; k++) hc[k] = ctx->lanes[0].h_mail[8 + k];
   ctx->d2h_bytes += (4 * P + 1) * 8;
   if (hc[4 * P] == 2) { set_error("exchange: timed out waiting for a peer's flag (a replica did not reach this exchange)"); return DBSP_ERR_CUDA; }
   if (hc[4 * P] != 0) {
@@ -581,20 +583,21 @@ int32_t comm_exchange(Ctx* ctx, const Batch* const* in, int ns, int fixed_dest, 
 
 int32_t comm_allreduce_max(Ctx* ctx, u64* x) {
   Comm* c = ctx->comm;
+  if (t_lane != 0 || ctx->fork_open) { set_error("allreduce: called inside a fork of the execution lanes"); return DBSP_ERR_INVALID; }
   if (!c || c->world == 1) return DBSP_OK;
   if (!c->connected) { set_error("allreduce: dbsp_comm_connect has not been called"); return DBSP_ERR_INVALID; }
   const u64 seq = ++c->red_seq;
   const int par = (int)(seq & 1);
   RedArgs ra;
   for (int p = 0; p < c->world; p++) ra.slot[p] = &((Ctrl*)c->peer[p])->red[par][c->rank];
-  const u64 mseq = ++ctx->mail_seq;
-  k_comm_allreduce_max<<<1, 32, 0, ctx->stream>>>(ra, ((Ctrl*)c->region)->red[par], (u32)c->world, *x, seq,
-                                                                        (volatile u64*)ctx->d_mail, mseq, comm_timeout_ns());
+  const u64 mseq = ++ctx->lanes[0].mail_seq;
+  k_comm_allreduce_max<<<1, 32, 0, ctx->lanes[0].stream>>>(ra, ((Ctrl*)c->region)->red[par], (u32)c->world, *x, seq,
+                                                                        (volatile u64*)ctx->lanes[0].d_mail, mseq, comm_timeout_ns());
   ctx->kernel_launches++;
   TRY(mail_wait(ctx, mseq));
-  ctx->n_sync++;
-  if (ctx->h_mail[9] != 0) { set_error("allreduce: timed out waiting for a peer"); return DBSP_ERR_CUDA; }
-  *x = ctx->h_mail[8];
+  ctx->lanes[0].n_sync++;
+  if (ctx->lanes[0].h_mail[9] != 0) { set_error("allreduce: timed out waiting for a peer"); return DBSP_ERR_CUDA; }
+  *x = ctx->lanes[0].h_mail[8];
   return DBSP_OK;
 }
 

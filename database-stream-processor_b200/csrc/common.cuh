@@ -9,9 +9,12 @@
 #include <stdint.h>
 
 #include <atomic>
+#include <functional>
 #include <map>
+#include <mutex>
 #include <memory>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "../../include/dbsp_b200.h"
@@ -112,7 +115,7 @@ struct Spine {
   Ctx* ctx = nullptr;
 };
 
-// Kernel ids for the optional per-kernel timing (CUDA events on the context's
+// Kernel ids for the optional per-kernel timing (CUDA events on the lane's
 // stream; bench.py's roofline figures come from here).
 enum KernelId {
   KID_MERGE = 0, KID_MERGE_PARTITION, KID_PROBE_RANGES, KID_PROBE_FILL, KID_PROJECT, KID_RADIX_SORT, KID_PACK,
@@ -124,51 +127,80 @@ struct ProfRec {
   u64 bytes;
 };
 
+// An execution lane: a compute stream with its own scratch words, mailbox slot and timing records.  Lane 0 is the
+// context's main stream; lane 1 runs the independent half of a grouped call (dbsp_join_step,
+// dbsp_batches_from_tables) on a worker thread between a fork and a join.  The host thread that drives a lane reads
+// it through lane(ctx), so the operator code is the same on both.
+struct Lane {
+  cudaStream_t stream = nullptr;
+  u64* d_scratch = nullptr;         // 256 u64
+  volatile u64* h_mail = nullptr;   // zero-copy mailbox: [0] = sequence flag, [8..] = payload (mapped pinned, 320 u64)
+  u64* d_mail = nullptr;            // its device alias
+  u64 mail_seq = 0;
+  cudaEvent_t ev = nullptr;         // fork (lane 0) / join (lane 1) point
+  u64 n_sync = 0;
+  double t_sync_us = 0;
+  std::vector<ProfRec> prof;
+  std::vector<cudaEvent_t> ev_pool;
+};
+constexpr int N_LANES = 2;
+struct LaneWorker;
+
 struct Ctx {
   // lifetime: device buffers may outlive dbsp_ctx_destroy (host handles are
   // freed by a garbage collector); the struct is deleted with the last buffer.
   std::atomic<long> live_bufs{0};
   bool destroyed = false;
   bool prof_on = false;
-  std::vector<ProfRec> prof;
-  std::vector<cudaEvent_t> ev_pool;
   int device = 0;
-  cudaStream_t stream = nullptr;
+  Lane lanes[N_LANES];
   cudaStream_t copy_stream = nullptr;   // pipelined H2D uploads (dbsp_upload_begin)
   cudaStream_t read_stream = nullptr;   // asynchronous D2H reads (dbsp_batch_download_begin): PCIe is full duplex
-  // pinned scratch for small D2H readbacks (counts, min/max)
+  // pinned scratch for small D2H readbacks (counts, min/max); lane 0 only
   u64* h_scratch = nullptr;   // 256 u64
-  // zero-copy mailbox for small read-backs: [0] = sequence flag, [8..] = payload
-  volatile u64* h_mail = nullptr;   // mapped pinned host memory (320 u64)
-  u64* d_mail = nullptr;            // its device alias
-  u64 mail_seq = 0;
-  u64* d_scratch = nullptr;   // 256 u64
-  u64 kernel_launches = 0, h2d_bytes = 0, d2h_bytes = 0;
+  std::atomic<u64> kernel_launches{0}, h2d_bytes{0}, d2h_bytes{0};
   // Device memory: best-fit allocator with coalescing over large cudaMalloc
-  // slabs.  Everything runs on one stream, so a block freed by the host can be
-  // handed out again at once: later work is ordered after the work that last
-  // touched it.  (The stream-ordered cudaMallocAsync pool cost ~25 ms/step in
-  // pool growth on q4; a cudaMalloc per slab costs ~10 ms, so slabs are big.)
+  // slabs.  Outside a fork everything runs on lane 0's stream, so a block freed
+  // by the host can be handed out again at once: later work is ordered after the
+  // work that last touched it.  Inside a fork the two lanes are not ordered
+  // against each other: blocks freed then wait in `pending_free` until the join
+  // has made lane 0 wait for lane 1.  (The stream-ordered cudaMallocAsync pool
+  // cost ~25 ms/step in pool growth on q4; a cudaMalloc per slab costs ~10 ms,
+  // so slabs are big.)
+  std::mutex pool_mu;                          // guards everything below up to n_alloc
+  bool fork_open = false;
+  std::vector<std::pair<char*, size_t>> pending_free;
   std::map<char*, size_t> free_by_addr;        // free blocks, for coalescing
   std::multimap<size_t, char*> free_by_size;   // the same blocks, for best fit
   std::map<char*, size_t> slabs;               // slab start -> bytes
   size_t pool_reserved = 0, pool_free = 0;
   // host-side overhead counters (printed at destroy when DBSP_HOST_STATS is set)
-  double t_alloc_us = 0, t_sync_us = 0;
-  u64 n_alloc = 0, n_sync = 0;
+  double t_alloc_us = 0;
+  u64 n_alloc = 0;
   int sm_count = 148;
   Comm* comm = nullptr;   // exchange state (comm.cu), owned by the context
+  LaneWorker* worker = nullptr;   // drives lane 1; created on the first fork
 };
+
+// The lane the calling thread drives: lane 1 on a context's worker thread, lane 0 everywhere else.
+extern thread_local int t_lane;
+inline Lane& lane(Ctx* c) { return c->lanes[t_lane]; }
+
+// Run `a` on lane 0 (this thread) and `b` on lane 1 (the worker thread) after the work queued so far on lane 0;
+// returns once both have been queued and lane 0 waits for lane 1.  The status is a's if it failed, else b's
+// (with b's error message).
+int32_t run_forked(Ctx* ctx, const std::function<int32_t()>& a, const std::function<int32_t()>& b);
+void lanes_shutdown(Ctx* ctx);
 
 #define LAUNCH_COUNT(ctx) ((ctx)->kernel_launches++)
 
 // RAII timing scope: records events around the kernels launched inside it.
 struct ProfScope {
-  Ctx* c;
+  Lane* l;
   long idx = -1;
   ProfScope(Ctx* ctx, int id, u64 bytes);
   ~ProfScope();
-  void set_bytes(u64 b) { if (idx >= 0) c->prof[idx].bytes = b; }
+  void set_bytes(u64 b) { if (idx >= 0) l->prof[idx].bytes = b; }
 };
 const char* kernel_name(int id);
 

@@ -488,7 +488,7 @@ int32_t consolidate_rows(Ctx* ctx, const dbsp_schema& s, const Cols& cols, const
   const int L = s.n_key_lanes + s.n_val_lanes;
   if (n == 0) { *out = batch_new_empty(ctx, s); return DBSP_OK; }   // with d_n: n is an upper bound
   if (n >= (1ull << 32)) { set_error("consolidate: more than 2^32-1 rows in one batch"); return DBSP_ERR_UNSUPPORTED; }
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = lane(ctx).stream;
   const int TB = 256;
 
   Flips f;
@@ -497,7 +497,7 @@ int32_t consolidate_rows(Ctx* ctx, const dbsp_schema& s, const Cols& cols, const
   // ---- (1) lane ranges + order / duplicate / zero-weight census ---------------
   u64 mm[2 * MAXL + 6];
   {
-    u64* dmm = ctx->d_scratch + 64;
+    u64* dmm = lane(ctx).d_scratch + 64;
     k_init_props<<<1, 32, 0, st>>>(dmm, L);
     const Mail mail = mail_begin(ctx);
     int g = (int)std::min<u64>((n + TB - 1) / TB, (u64)ctx->sm_count * 8);
@@ -598,7 +598,7 @@ int32_t consolidate_rows(Ctx* ctx, const dbsp_schema& s, const Cols& cols, const
   u64* const kbufs[2] = {kbuf ? (u64*)kbuf->p : nullptr, kbuf ? (u64*)kbuf->p + n : nullptr};
   u64* const k1bufs[2] = {(kbuf && p.W == 2) ? (u64*)kbuf->p + 2 * n : nullptr, (kbuf && p.W == 2) ? (u64*)kbuf->p + 3 * n : nullptr};
   u32* const ibufs[2] = {ibuf ? (u32*)ibuf->p : nullptr, ibuf ? (u32*)ibuf->p + n : nullptr};
-  u64* const cnt = ctx->d_scratch + 32;   // [0] output rows, [2] sort-fallback flag
+  u64* const cnt = lane(ctx).d_scratch + 32;   // [0] output rows, [2] sort-fallback flag
   const u64* key1_sorted = nullptr;
   // lane 0 ordered on arrival (event tables come in time order): the top bits[0] bits of the key are non-decreasing
   // already, the sort needs no HBM pass (sort.cu)
@@ -709,7 +709,7 @@ int32_t reduce_sorted_rows(Ctx* ctx, const dbsp_schema& s, const Cols& cols, con
   const int L = s.n_key_lanes + s.n_val_lanes;
   if (n == 0) { *out = batch_new_empty(ctx, s); return DBSP_OK; }
   if (n >= (1ull << 32)) { set_error("reduce: more than 2^32-1 rows in one batch"); return DBSP_ERR_UNSUPPORTED; }
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = lane(ctx).stream;
   Plan p;
   memset(&p, 0, sizeof(p));
   p.L = L;
@@ -721,7 +721,7 @@ int32_t reduce_sorted_rows(Ctx* ctx, const dbsp_schema& s, const Cols& cols, con
   TRY(dev_alloc(ctx, (size_t)ntiles * sizeof(ReStatus) + 16, &tbuf));
   ReStatus* status = (ReStatus*)tbuf->p;
   u32* ticket = (u32*)(status + ntiles);
-  u64* const cnt = ctx->d_scratch + 32;
+  u64* const cnt = lane(ctx).d_scratch + 32;
   Batch* b = nullptr;
   MCols oc;
   i64* ow;

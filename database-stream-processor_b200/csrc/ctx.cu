@@ -3,6 +3,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <condition_variable>
 #include <iterator>
 #include <cstdio>
 #include <cstdlib>
@@ -14,12 +15,14 @@ static inline double now_us() {
 }
 
 static thread_local std::string g_err;
+thread_local int t_lane = 0;
 void set_error(const std::string& s) { g_err = s; }
 void print_host_stats(Ctx* c) {
   if (getenv("DBSP_HOST_STATS"))
-    fprintf(stderr, "[dbsp host] allocs %llu in %.1f ms (pool %.2f GiB in %zu slabs); read-back syncs %llu waited %.1f ms; launches %llu\n",
-            (unsigned long long)c->n_alloc, c->t_alloc_us / 1e3, c->pool_reserved / 1073741824.0, c->slabs.size(), (unsigned long long)c->n_sync, c->t_sync_us / 1e3,
-            (unsigned long long)c->kernel_launches);
+    fprintf(stderr, "[dbsp host] allocs %llu in %.1f ms (pool %.2f GiB in %zu slabs); read-back syncs %llu + %llu waited %.1f + %.1f ms (lane 0 + 1); launches %llu\n",
+            (unsigned long long)c->n_alloc, c->t_alloc_us / 1e3, c->pool_reserved / 1073741824.0, c->slabs.size(),
+            (unsigned long long)c->lanes[0].n_sync, (unsigned long long)c->lanes[1].n_sync, c->lanes[0].t_sync_us / 1e3,
+            c->lanes[1].t_sync_us / 1e3, (unsigned long long)c->kernel_launches.load());
 }
 const char* get_error() { return g_err.c_str(); }
 
@@ -28,21 +31,21 @@ static const char* KNAMES[KID_COUNT] = {
     "heads", "emit", "minmax", "seg_reduce", "lookup", "compact", "scan", "agg_pick", "misc", "shard_scatter", "chunk_sort"};
 const char* kernel_name(int id) { return (id >= 0 && id < KID_COUNT) ? KNAMES[id] : "?"; }
 
-ProfScope::ProfScope(Ctx* ctx, int id, u64 bytes) : c(ctx) {
+ProfScope::ProfScope(Ctx* ctx, int id, u64 bytes) : l(&lane(ctx)) {
   if (!ctx->prof_on) return;
   ProfRec r;
   r.id = id;
   r.bytes = bytes;
   for (cudaEvent_t* e : {&r.a, &r.b}) {
-    if (!ctx->ev_pool.empty()) { *e = ctx->ev_pool.back(); ctx->ev_pool.pop_back(); }
+    if (!l->ev_pool.empty()) { *e = l->ev_pool.back(); l->ev_pool.pop_back(); }
     else cudaEventCreate(e);
   }
-  cudaEventRecord(r.a, ctx->stream);
-  idx = (long)ctx->prof.size();
-  ctx->prof.push_back(r);
+  cudaEventRecord(r.a, l->stream);
+  idx = (long)l->prof.size();
+  l->prof.push_back(r);
 }
 ProfScope::~ProfScope() {
-  if (idx >= 0) cudaEventRecord(c->prof[idx].b, c->stream);
+  if (idx >= 0) cudaEventRecord(l->prof[idx].b, l->stream);
 }
 
 static const size_t SLAB_BYTES = (size_t)8 << 30;   // 8 GiB per cudaMalloc
@@ -84,8 +87,13 @@ static void pool_insert_free(Ctx* ctx, char* p, size_t sz) {
 DevBuf::~DevBuf() {
   if (!ctx) return;
   if (p && !ctx->destroyed) {   // after ctx_destroy the slabs are already gone
-    pool_insert_free(ctx, (char*)p, cls);
-    ctx->pool_free += cls;
+    std::lock_guard<std::mutex> g(ctx->pool_mu);
+    if (ctx->fork_open) {   // the other lane may still use the block: free it at the join
+      ctx->pending_free.push_back({(char*)p, cls});
+    } else {
+      pool_insert_free(ctx, (char*)p, cls);
+      ctx->pool_free += cls;
+    }
   }
   if (ctx->live_bufs.fetch_sub(1) == 1 && ctx->destroyed) delete ctx;
 }
@@ -97,6 +105,7 @@ int32_t dev_alloc(Ctx* ctx, size_t bytes, BufP* out) {
   b->bytes = bytes;
   if (bytes == 0) bytes = 16;
   size_t need = (bytes + ALIGN - 1) & ~(ALIGN - 1);
+  std::lock_guard<std::mutex> g(ctx->pool_mu);
   double t0 = now_us();
   auto it = ctx->free_by_size.lower_bound(need);
   if (it == ctx->free_by_size.end()) {
@@ -175,6 +184,107 @@ void batch_unref(Batch* b) {
   if (b->refs.fetch_sub(1) == 1) delete b;
 }
 
+// ---- lane 1: a worker thread owned by the context ------------------------------------------------------------------
+// The worker spins while it expects a fork (the forks of one circuit step follow each other within a fraction of a
+// millisecond, and waking a parked thread costs about as much as one of the kernels the fork hides) and parks on a
+// condition variable once it has been idle for LANE_SPIN_US.
+static const double LANE_SPIN_US = 1000.0;
+enum { W_IDLE = 0, W_POSTED, W_DONE, W_EXIT };
+struct LaneWorker {
+  std::thread th;
+  std::mutex m;
+  std::condition_variable cv;
+  std::atomic<int> state{W_IDLE};
+  const std::function<int32_t()>* job = nullptr;
+  int32_t rc = DBSP_OK;
+  std::string err;
+};
+
+static inline void cpu_relax() {
+#if defined(__x86_64__) || defined(__i386__)
+  __builtin_ia32_pause();
+#else
+  std::this_thread::yield();
+#endif
+}
+
+static void lane_worker_main(Ctx* ctx, LaneWorker* w) {
+  t_lane = 1;
+  cudaSetDevice(ctx->device);
+  while (true) {
+    int st;
+    double t0 = now_us();
+    while ((st = w->state.load(std::memory_order_acquire)) != W_POSTED && st != W_EXIT) {
+      if (now_us() - t0 < LANE_SPIN_US) { cpu_relax(); continue; }
+      std::unique_lock<std::mutex> lk(w->m);
+      w->cv.wait(lk, [w] { int x = w->state.load(); return x == W_POSTED || x == W_EXIT; });
+    }
+    if (st == W_EXIT) return;
+    w->rc = (*w->job)();
+    w->err = w->rc != DBSP_OK ? std::string(get_error()) : std::string();
+    w->state.store(W_DONE, std::memory_order_release);
+  }
+}
+
+void lanes_shutdown(Ctx* ctx) {
+  LaneWorker* w = ctx->worker;
+  if (!w) return;
+  {
+    std::lock_guard<std::mutex> g(w->m);
+    w->state.store(W_EXIT);
+  }
+  w->cv.notify_one();
+  w->th.join();
+  delete w;
+  ctx->worker = nullptr;
+}
+
+int32_t run_forked(Ctx* ctx, const std::function<int32_t()>& a, const std::function<int32_t()>& b) {
+  if (t_lane != 0 || ctx->fork_open) { set_error("fork: already inside a fork"); return DBSP_ERR_INVALID; }
+  Lane& l0 = ctx->lanes[0];
+  Lane& l1 = ctx->lanes[1];
+  if (!ctx->worker) {
+    ctx->worker = new LaneWorker();
+    ctx->worker->th = std::thread(lane_worker_main, ctx, ctx->worker);
+  }
+  LaneWorker* w = ctx->worker;
+  // fork: lane 1 starts after everything queued on lane 0 so far
+  CUDA_TRY(cudaEventRecord(l0.ev, l0.stream));
+  CUDA_TRY(cudaStreamWaitEvent(l1.stream, l0.ev, 0));
+  {
+    std::lock_guard<std::mutex> g(ctx->pool_mu);
+    ctx->fork_open = true;
+  }
+  w->job = &b;
+  {
+    std::lock_guard<std::mutex> g(w->m);
+    w->state.store(W_POSTED, std::memory_order_release);
+  }
+  w->cv.notify_one();
+  const int32_t ra = a();
+  const std::string ea = ra != DBSP_OK ? std::string(get_error()) : std::string();
+  while (w->state.load(std::memory_order_acquire) != W_DONE) cpu_relax();
+  w->state.store(W_IDLE, std::memory_order_relaxed);
+  // join: lane 0 continues after everything lane 1 queued; only then may the blocks freed inside the fork be reused
+  cudaError_t e = cudaEventRecord(l1.ev, l1.stream);
+  if (e == cudaSuccess) e = cudaStreamWaitEvent(l0.stream, l1.ev, 0);
+  {
+    std::lock_guard<std::mutex> g(ctx->pool_mu);
+    ctx->fork_open = false;
+    if (e == cudaSuccess) {
+      for (auto& f : ctx->pending_free) {
+        pool_insert_free(ctx, f.first, f.second);
+        ctx->pool_free += f.second;
+      }
+      ctx->pending_free.clear();
+    }
+  }
+  if (e != cudaSuccess) { set_error(std::string("join of the lanes: ") + cudaGetErrorString(e)); return DBSP_ERR_CUDA; }
+  if (ra != DBSP_OK) { set_error(ea); return ra; }
+  if (w->rc != DBSP_OK) { set_error(w->err); return w->rc; }
+  return DBSP_OK;
+}
+
 // Small device->host read-backs (row counts, lane ranges).  A one-warp kernel
 // copies the words into mapped pinned host memory and then publishes a sequence
 // number; the host spins on that word.  This costs a few microseconds instead of
@@ -196,16 +306,17 @@ __global__ void k_publish(volatile u64* mail, const u64* src, int count, int wor
 }
 
 int32_t mail_wait(Ctx* ctx, u64 seq) {
+  Lane& ln = lane(ctx);
   u64 spins = 0;
-  while (ctx->h_mail[0] != seq) {
+  while (ln.h_mail[0] != seq) {
     if ((++spins & 0xffff) == 0) {   // the stream may have faulted: do not spin forever
-      cudaError_t e = cudaStreamQuery(ctx->stream);
+      cudaError_t e = cudaStreamQuery(ln.stream);
       if (e != cudaSuccess && e != cudaErrorNotReady) {
         set_error(std::string("read_back: ") + cudaGetErrorString(e));
         return DBSP_ERR_CUDA;
       }
-      if (e == cudaSuccess && ctx->h_mail[0] != seq) {   // kernel done but the flag is not visible yet
-        CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+      if (e == cudaSuccess && ln.h_mail[0] != seq) {   // kernel done but the flag is not visible yet
+        CUDA_TRY(cudaStreamSynchronize(ln.stream));
       }
     }
   }
@@ -213,42 +324,46 @@ int32_t mail_wait(Ctx* ctx, u64 seq) {
 }
 
 Mail mail_begin(Ctx* ctx) {
+  Lane& ln = lane(ctx);
   Mail m;
-  m.p = (volatile u64*)ctx->d_mail;
-  m.seq = ++ctx->mail_seq;
+  m.p = (volatile u64*)ln.d_mail;
+  m.seq = ++ln.mail_seq;
   return m;
 }
 int32_t mail_finish(Ctx* ctx, const Mail& m, u64* out, int count) {
+  Lane& ln = lane(ctx);
   double t0 = now_us();
   TRY(mail_wait(ctx, m.seq));
-  ctx->t_sync_us += now_us() - t0;
-  ctx->n_sync++;
-  for (int i = 0; i < count; i++) out[i] = ctx->h_mail[8 + i];
+  ln.t_sync_us += now_us() - t0;
+  ln.n_sync++;
+  for (int i = 0; i < count; i++) out[i] = ln.h_mail[8 + i];
   ctx->d2h_bytes += (u64)count * 8;
   return DBSP_OK;
 }
 
 int32_t read_back(Ctx* ctx, const void* dsrc, size_t count_u64, u64* hdst) {
   if (count_u64 > 256) { set_error("read_back: too large"); return DBSP_ERR_INVALID; }
+  Lane& ln = lane(ctx);
   double t0 = now_us();
-  const u64 seq = ++ctx->mail_seq;
-  k_publish<<<1, 32, 0, ctx->stream>>>((volatile u64*)ctx->d_mail, (const u64*)dsrc, (int)count_u64, 0, seq);
+  const u64 seq = ++ln.mail_seq;
+  k_publish<<<1, 32, 0, ln.stream>>>((volatile u64*)ln.d_mail, (const u64*)dsrc, (int)count_u64, 0, seq);
   TRY(mail_wait(ctx, seq));
-  ctx->t_sync_us += now_us() - t0;
-  ctx->n_sync++;
-  for (size_t i = 0; i < count_u64; i++) hdst[i] = ctx->h_mail[8 + i];
+  ln.t_sync_us += now_us() - t0;
+  ln.n_sync++;
+  for (size_t i = 0; i < count_u64; i++) hdst[i] = ln.h_mail[8 + i];
   ctx->d2h_bytes += count_u64 * 8;
   return DBSP_OK;
 }
 
 int32_t read_back32(Ctx* ctx, const void* dsrc, u32* hdst) {
+  Lane& ln = lane(ctx);
   double t0 = now_us();
-  const u64 seq = ++ctx->mail_seq;
-  k_publish<<<1, 32, 0, ctx->stream>>>((volatile u64*)ctx->d_mail, (const u64*)dsrc, 1, 1, seq);
+  const u64 seq = ++ln.mail_seq;
+  k_publish<<<1, 32, 0, ln.stream>>>((volatile u64*)ln.d_mail, (const u64*)dsrc, 1, 1, seq);
   TRY(mail_wait(ctx, seq));
-  ctx->t_sync_us += now_us() - t0;
-  ctx->n_sync++;
-  *hdst = (u32)ctx->h_mail[8];
+  ln.t_sync_us += now_us() - t0;
+  ln.n_sync++;
+  *hdst = (u32)ln.h_mail[8];
   ctx->d2h_bytes += 4;
   return DBSP_OK;
 }
@@ -346,7 +461,7 @@ int32_t exclusive_scan_u32(Ctx* ctx, const u32* in, u32* out, u64 n, const Mail*
   const u32 ntiles = (u32)((m + SCAN_TILE - 1) / SCAN_TILE);
   BufP aux;
   TRY(dev_alloc(ctx, (size_t)(ntiles + 1) * 8, &aux));
-  CUDA_TRY(cudaMemsetAsync(aux->p, 0, (size_t)(ntiles + 1) * 8, ctx->stream));
+  CUDA_TRY(cudaMemsetAsync(aux->p, 0, (size_t)(ntiles + 1) * 8, lane(ctx).stream));
   u64* status = (u64*)aux->p;
   u32* ticket = (u32*)(status + ntiles);
   {
@@ -355,7 +470,7 @@ int32_t exclusive_scan_u32(Ctx* ctx, const u32* in, u32* out, u64 n, const Mail*
     mm.p = nullptr;
     mm.seq = 0;
     if (total_mail) mm = *total_mail;
-    k_exscan_u32<<<ntiles, SCAN_THREADS, 0, ctx->stream>>>(in, out, m, ticket, status, mm);
+    k_exscan_u32<<<ntiles, SCAN_THREADS, 0, lane(ctx).stream>>>(in, out, m, ticket, status, mm);
   }
   LAUNCH_COUNT(ctx);
   return DBSP_OK;
@@ -365,10 +480,10 @@ int32_t exclusive_scan_u32(Ctx* ctx, const u32* in, u32* out, u64 n, const Mail*
 // one library prefix sum left.
 int32_t inclusive_scan_i64(Ctx* ctx, const i64* in, i64* out, u64 n) {
   size_t tmp_bytes = 0;
-  CUDA_TRY(cub::DeviceScan::InclusiveSum(nullptr, tmp_bytes, in, out, (size_t)n, ctx->stream));
+  CUDA_TRY(cub::DeviceScan::InclusiveSum(nullptr, tmp_bytes, in, out, (size_t)n, lane(ctx).stream));
   BufP tmp;
   TRY(dev_alloc(ctx, tmp_bytes, &tmp));
-  CUDA_TRY(cub::DeviceScan::InclusiveSum(tmp->p, tmp_bytes, in, out, (size_t)n, ctx->stream));
+  CUDA_TRY(cub::DeviceScan::InclusiveSum(tmp->p, tmp_bytes, in, out, (size_t)n, lane(ctx).stream));
   LAUNCH_COUNT(ctx);
   return DBSP_OK;
 }

@@ -648,7 +648,7 @@ bool uniform_phase(const Batch* b) {
 template <int L>
 int32_t merge_launch(Ctx* ctx, const Batch* a, const Batch* b, Batch** out) {
   typedef MergeCfg<L> Cfg;
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = lane(ctx).stream;
   u64 total = a->n + b->n;
   u32 ntiles = (u32)((total + Cfg::TILE - 1) / Cfg::TILE);
   BufP aux;
@@ -683,7 +683,7 @@ int32_t merge_launch(Ctx* ctx, const Batch* a, const Batch* b, Batch** out) {
   int32_t rc = mail_finish(ctx, mail, &nout, 1);
   if (rc != DBSP_OK) { batch_unref(o); return rc; }
   // algorithmic bytes: every input row read once, every output row written once
-  if (ps_idx >= 0) ctx->prof[ps_idx].bytes = (total + nout) * (u64)(L + 1) * 8;
+  if (ps_idx >= 0) lane(ctx).prof[ps_idx].bytes = (total + nout) * (u64)(L + 1) * 8;
   o->n = nout;
   if (nout == 0) { batch_unref(o); o = batch_new_empty(ctx, a->s); }
   *out = o;
@@ -692,8 +692,8 @@ int32_t merge_launch(Ctx* ctx, const Batch* a, const Batch* b, Batch** out) {
 
 template <int L>
 int32_t split_launch(Ctx* ctx, const Batch* a, const Batch* b, u64 d, u64* na, u64* nb) {
-  u64* dout = ctx->d_scratch + 124;
-  k_merge_split<L><<<1, 1, 0, ctx->stream>>>(a->cols(), a->n, b->cols(), b->n, a->flips(), d, dout);
+  u64* dout = lane(ctx).d_scratch + 124;
+  k_merge_split<L><<<1, 1, 0, lane(ctx).stream>>>(a->cols(), a->n, b->cols(), b->n, a->flips(), d, dout);
   ctx->kernel_launches++;
   u64 h[2];
   TRY(read_back(ctx, dout, 2, h));

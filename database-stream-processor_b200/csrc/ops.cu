@@ -834,7 +834,7 @@ int32_t compact_ordered(Ctx* ctx, const dbsp_schema& s, const Cols& in, const i6
   MCols oc;
   i64* ow;
   TRY(batch_alloc(ctx, s, nout, &b, &oc, &ow));
-  k_scatter<<<blocks(n), TB, 0, ctx->stream>>>(in, L, w, keep, pos, n, oc, ow);
+  k_scatter<<<blocks(n), TB, 0, lane(ctx).stream>>>(in, L, w, keep, pos, n, oc, ow);
   LAUNCH_COUNT(ctx);
   *out = b;
   return DBSP_OK;
@@ -856,7 +856,7 @@ int32_t op_truncate_values(Ctx* ctx, const Batch* b, const u64* val_bound, Batch
   u32* pos = keep + (n + 1);
   {
     ProfScope ps(ctx, KID_COMPACT, n * (u64)nv * 8);
-    k_vals_ge<<<blocks(n + 1), TB, 0, ctx->stream>>>(b->cols(), n, nk, nv, rb, f, keep);
+    k_vals_ge<<<blocks(n + 1), TB, 0, lane(ctx).stream>>>(b->cols(), n, nk, nv, rb, f, keep);
   }
   LAUNCH_COUNT(ctx);
   const Mail mail = mail_begin(ctx);
@@ -872,7 +872,7 @@ int32_t op_truncate_values(Ctx* ctx, const Batch* b, const u64* val_bound, Batch
   TRY(batch_alloc(ctx, b->s, nout, &o, &oc, &ow));
   {
     ProfScope ps(ctx, KID_COMPACT, (n + nout) * (u64)(b->nl() + 1) * 8);
-    k_scatter<<<blocks(n), TB, 0, ctx->stream>>>(b->cols(), b->nl(), b->w, keep, pos, n, oc, ow);
+    k_scatter<<<blocks(n), TB, 0, lane(ctx).stream>>>(b->cols(), b->nl(), b->w, keep, pos, n, oc, ow);
   }
   LAUNCH_COUNT(ctx);
   *out = o;
@@ -913,8 +913,8 @@ int32_t batch_concat(Ctx* ctx, const dbsp_schema& s, std::vector<Batch*>& parts,
   u64 off = 0;
   for (Batch* p : live) {
     for (int l = 0; l < L; l++)
-      cudaMemcpyAsync(oc.c[l] + off, p->col[l], p->n * 8, cudaMemcpyDeviceToDevice, ctx->stream);
-    cudaMemcpyAsync(ow + off, p->w, p->n * 8, cudaMemcpyDeviceToDevice, ctx->stream);
+      cudaMemcpyAsync(oc.c[l] + off, p->col[l], p->n * 8, cudaMemcpyDeviceToDevice, lane(ctx).stream);
+    cudaMemcpyAsync(ow + off, p->w, p->n * 8, cudaMemcpyDeviceToDevice, lane(ctx).stream);
     off += p->n;
     batch_unref(p);
   }
@@ -958,7 +958,7 @@ int32_t project_and_consolidate(Ctx* ctx, const Cols& in, int nk_in, int n_in_la
   if (filtered) {
     // status[g] u64 | ticket u32, surviving-row count u32
     TRY(dev_alloc(ctx, (size_t)(g + 1) * 8, &cb));
-    CUDA_TRY(cudaMemsetAsync(cb->p, 0, (size_t)(g + 1) * 8, ctx->stream));
+    CUDA_TRY(cudaMemsetAsync(cb->p, 0, (size_t)(g + 1) * 8, lane(ctx).stream));
     status = (u64*)cb->p;
     ticket = (u32*)(status + g);
     d_mw = ticket + 1;   // stays on the device; the census of consolidate_rows returns it
@@ -969,7 +969,7 @@ int32_t project_and_consolidate(Ctx* ctx, const Cols& in, int nk_in, int n_in_la
   {
     // the lanes the closure names read once, the output rows written once (bound: every row survives)
     ProfScope ps(ctx, KID_PROJECT, n * (u64)(used_lanes(proj, n_in_lanes, nk_in) + (w ? 1 : 0)) * 8 + m * (u64)(Lo + 1) * 8);
-    k_project_rows<<<g, TB, 0, ctx->stream>>>(in, nk_in, w, n, proj, filtered ? 0 : 1, g, ticket, status, t.c, t.w, d_mw);
+    k_project_rows<<<g, TB, 0, lane(ctx).stream>>>(in, nk_in, w, n, proj, filtered ? 0 : 1, g, ticket, status, t.c, t.w, d_mw);
   }
   LAUNCH_COUNT(ctx);
   return consolidate_rows(ctx, os, t.cc(), t.w, m, &t.buf, out, d_m);
@@ -979,7 +979,7 @@ int32_t project_and_consolidate(Ctx* ctx, const Cols& in, int nk_in, int n_in_la
 // proj == nullptr: gather the matching trace rows unchanged.
 static int32_t probe_chunk(Ctx* ctx, const Batch* delta, int nk, Batch* const* tb, int nb, const dbsp_proj* proj,
                            int delta_is_left, const dbsp_schema& out_schema, Batch** out) {
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = lane(ctx).stream;
   const u64 nd = delta->n;
   Flips f = delta->flips();
   BatchRefs refs;
@@ -1089,7 +1089,7 @@ static int32_t distinct_keys(Ctx* ctx, const Batch* b, int nk, Batch** out) {
   BufP fb;
   TRY(dev_alloc(ctx, (size_t)(b->n + 1) * 4, &fb));
   u32* flags = (u32*)fb->p;
-  k_key_heads<<<blocks(b->n + 1), TB, 0, ctx->stream>>>(b->cols(), b->n, nk, flags);
+  k_key_heads<<<blocks(b->n + 1), TB, 0, lane(ctx).stream>>>(b->cols(), b->n, nk, flags);
   LAUNCH_COUNT(ctx);
   return compact_ordered(ctx, ks, b->cols(), b->w, flags, b->n, out);
 }
@@ -1097,7 +1097,7 @@ static int32_t distinct_keys(Ctx* ctx, const Batch* b, int nk, Batch** out) {
 // AggregateIncremental::eval + Upsert::eval
 // (operator/aggregate/mod.rs:479-547,600-684; operator/upsert.rs:161-208).
 int32_t op_aggregate_delta(Ctx* ctx, const Batch* delta, const Spine* in_tr, const Spine* out_tr, int kind, Batch** out) {
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = lane(ctx).stream;
   const dbsp_schema& os = out_tr->s;
   int nk = os.n_key_lanes, nov = os.n_val_lanes;
   if (delta->n == 0) { *out = batch_new_empty(ctx, os); return DBSP_OK; }
@@ -1122,7 +1122,7 @@ int32_t op_aggregate_delta(Ctx* ctx, const Batch* delta, const Spine* in_tr, con
     TRY(dev_alloc(ctx, (size_t)(keys->n + 1) * 4, &kb));
     TmpRows nvr;
     TRY(tmp_alloc(ctx, nov, keys->n, &nvr));
-    u64* slow = ctx->d_scratch + 16;
+    u64* slow = lane(ctx).d_scratch + 16;
     CUDA_TRY(cudaMemsetAsync(slow, 0, 8, st));
     {
       u64 lg = 1; while ((1ull << lg) < in_tr->batches[0]->n + 1) lg++;
@@ -1206,7 +1206,7 @@ int32_t op_neg(Ctx* ctx, const Batch* a, Batch** out) {
   if (a->n == 0) { *out = batch_new_empty(ctx, a->s); return DBSP_OK; }
   BufP wb;
   TRY(dev_alloc(ctx, (size_t)a->n * 8, &wb));
-  k_neg<<<blocks(a->n), TB, 0, ctx->stream>>>(a->w, a->n, (i64*)wb->p);
+  k_neg<<<blocks(a->n), TB, 0, lane(ctx).stream>>>(a->w, a->n, (i64*)wb->p);
   LAUNCH_COUNT(ctx);
   Batch* b = new Batch();
   b->s = a->s;
@@ -1232,7 +1232,7 @@ int32_t op_weigh(Ctx* ctx, const Batch* b, const dbsp_expr* f, int mode, Batch**
   ROWS32(m, "weigh");
   TmpRows t;
   TRY(tmp_alloc(ctx, os.n_key_lanes, m, &t));
-  k_weigh<<<blocks(b->n), TB, 0, ctx->stream>>>(b->cols(), b->w, b->n, nk, nv, *f, mode, t.c, t.w);
+  k_weigh<<<blocks(b->n), TB, 0, lane(ctx).stream>>>(b->cols(), b->w, b->n, nk, nv, *f, mode, t.c, t.w);
   LAUNCH_COUNT(ctx);
   return consolidate_rows(ctx, os, t.cc(), t.w, m, &t.buf, out);
 }
@@ -1241,7 +1241,7 @@ int32_t op_weigh(Ctx* ctx, const Batch* b, const dbsp_expr* f, int mode, Batch**
 int32_t op_distinct_delta(Ctx* ctx, const Batch* delta, const Spine* integral, Batch** out) {
   u64 n = delta->n;
   if (n == 0) { *out = batch_new_empty(ctx, delta->s); return DBSP_OK; }
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = lane(ctx).stream;
   BufP ab, kb;
   TRY(dev_alloc(ctx, (size_t)n * 8 * 2, &ab));
   TRY(dev_alloc(ctx, (size_t)(n + 1) * 4, &kb));
@@ -1264,7 +1264,7 @@ int32_t op_stream_distinct(Ctx* ctx, const Batch* b, Batch** out) {
   BufP ab, kb;
   TRY(dev_alloc(ctx, (size_t)n * 8, &ab));
   TRY(dev_alloc(ctx, (size_t)(n + 1) * 4, &kb));
-  k_positive<<<blocks(n + 1), TB, 0, ctx->stream>>>(b->w, n, (u32*)kb->p, (i64*)ab->p);
+  k_positive<<<blocks(n + 1), TB, 0, lane(ctx).stream>>>(b->w, n, (u32*)kb->p, (i64*)ab->p);
   LAUNCH_COUNT(ctx);
   return compact_ordered(ctx, b->s, b->cols(), (i64*)ab->p, (u32*)kb->p, n, out);
 }
@@ -1280,7 +1280,7 @@ int32_t op_semijoin(Ctx* ctx, const Batch* pairs, const Batch* keys, Batch** out
   BufP ab, kb;
   TRY(dev_alloc(ctx, (size_t)n * 8, &ab));
   TRY(dev_alloc(ctx, (size_t)(n + 1) * 4, &kb));
-  k_semijoin<<<blocks(n + 1), TB, 0, ctx->stream>>>(pairs->cols(), pairs->w, n, keys->cols(), keys->w, keys->n,
+  k_semijoin<<<blocks(n + 1), TB, 0, lane(ctx).stream>>>(pairs->cols(), pairs->w, n, keys->cols(), keys->w, keys->n,
                                                    pairs->s.n_key_lanes, pairs->flips(), (u32*)kb->p, (i64*)ab->p);
   LAUNCH_COUNT(ctx);
   return compact_ordered(ctx, os, pairs->cols(), (i64*)ab->p, (u32*)kb->p, n, out);
@@ -1311,7 +1311,7 @@ static int32_t merge_tree(Ctx* ctx, std::vector<Batch*>& parts, const dbsp_schem
 // Window::eval (operator/time_series/window.rs:144-222)
 int32_t op_window_delta(Ctx* ctx, const Spine* trace, const Batch* delta, int has_prev, const u64* s0, const u64* e0,
                         const u64* s1, const u64* e1, Batch** out) {
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = lane(ctx).stream;
   const dbsp_schema& s = delta->s;
   int nk = s.n_key_lanes, L = delta->nl();
   auto lt = [&](const u64* a, const u64* b) {
@@ -1404,16 +1404,16 @@ int32_t op_shard_partition(Ctx* ctx, const Batch* b, u32 P, Batch** outs) {
   TRY(dev_alloc(ctx, (size_t)(m + 1) * 4 * 2, &fb));
   u32* flags = (u32*)fb->p;
   u32* pos = flags + (m + 1);
-  k_shard_flags<<<blocks(n + 1), TB, 0, ctx->stream>>>(b->cols(), n, b->s.n_key_lanes, P, flags);
+  k_shard_flags<<<blocks(n + 1), TB, 0, lane(ctx).stream>>>(b->cols(), n, b->s.n_key_lanes, P, flags);
   LAUNCH_COUNT(ctx);
-  CUDA_TRY(cudaMemsetAsync(flags + m, 0, 4, ctx->stream));
+  CUDA_TRY(cudaMemsetAsync(flags + m, 0, 4, lane(ctx).stream));
   TRY(exclusive_scan_u32(ctx, flags, pos, m));
   Batch* all;   // one buffer holding the P shards back to back; the shards are views
   MCols oc;
   i64* ow;
   TRY(batch_alloc(ctx, b->s, n, &all, &oc, &ow));
-  u64* bounds = ctx->d_scratch + 160;
-  k_shard_scatter<<<blocks(std::max<u64>(n, P + 1)), TB, 0, ctx->stream>>>(b->cols(), L, b->w, flags, pos, n, P, oc, ow, bounds);
+  u64* bounds = lane(ctx).d_scratch + 160;
+  k_shard_scatter<<<blocks(std::max<u64>(n, P + 1)), TB, 0, lane(ctx).stream>>>(b->cols(), L, b->w, flags, pos, n, P, oc, ow, bounds);
   LAUNCH_COUNT(ctx);
   u64 hb[65];
   int32_t rc = read_back(ctx, bounds, P + 1, hb);
@@ -1444,7 +1444,7 @@ int32_t batch_build_csr(Ctx* ctx, Batch* b) {
   TRY(dev_alloc(ctx, (size_t)(b->n + 1) * 4 * 2, &fb));
   u32* flags = (u32*)fb->p;
   u32* pos = flags + (b->n + 1);
-  k_key_heads<<<blocks(b->n + 1), TB, 0, ctx->stream>>>(b->cols(), b->n, nk, flags);
+  k_key_heads<<<blocks(b->n + 1), TB, 0, lane(ctx).stream>>>(b->cols(), b->n, nk, flags);
   LAUNCH_COUNT(ctx);
   const Mail mail = mail_begin(ctx);
   TRY(exclusive_scan_u32(ctx, flags, pos, b->n, &mail));
@@ -1452,7 +1452,7 @@ int32_t batch_build_csr(Ctx* ctx, Batch* b) {
   TRY(mail_finish(ctx, mail, &nkeys64, 1));
   const u32 nkeys = (u32)nkeys64;
   TRY(dev_alloc(ctx, (size_t)(nkeys + 1) * 8, &pb));
-  k_scatter_index<<<blocks(b->n), TB, 0, ctx->stream>>>(flags, pos, b->n, (u64*)pb->p, nkeys);
+  k_scatter_index<<<blocks(b->n), TB, 0, lane(ctx).stream>>>(flags, pos, b->n, (u64*)pb->p, nkeys);
   LAUNCH_COUNT(ctx);
   b->keystart = pb;
   b->nkeys = nkeys;
@@ -1464,10 +1464,10 @@ int32_t batch_lower_bound(Ctx* ctx, const Batch* b, const u64* key, u64* pos) {
   if (b->n == 0) { *pos = 0; return DBSP_OK; }
   u64 hq[MAXL] = {0};
   for (int l = 0; l < b->s.n_key_lanes; l++) hq[l] = key[l];
-  u64* dq = ctx->d_scratch + 96;
-  CUDA_TRY(cudaMemcpyAsync(dq, hq, sizeof(hq), cudaMemcpyHostToDevice, ctx->stream));
-  CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-  k_lower_bounds<<<1, 32, 0, ctx->stream>>>(b->cols(), b->n, b->s.n_key_lanes, b->flips(), dq, 1, ctx->d_scratch + 120);
+  u64* dq = lane(ctx).d_scratch + 96;
+  CUDA_TRY(cudaMemcpyAsync(dq, hq, sizeof(hq), cudaMemcpyHostToDevice, lane(ctx).stream));
+  CUDA_TRY(cudaStreamSynchronize(lane(ctx).stream));
+  k_lower_bounds<<<1, 32, 0, lane(ctx).stream>>>(b->cols(), b->n, b->s.n_key_lanes, b->flips(), dq, 1, lane(ctx).d_scratch + 120);
   LAUNCH_COUNT(ctx);
-  return read_back(ctx, ctx->d_scratch + 120, 1, pos);
+  return read_back(ctx, lane(ctx).d_scratch + 120, 1, pos);
 }

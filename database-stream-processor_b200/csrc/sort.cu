@@ -513,7 +513,7 @@ struct Bufs {   // the two ping-pong sets of a sort
 
 template <int W, bool BID>
 int32_t run_passes(Ctx* ctx, Bufs& B, int& cur, u64 n, const PassList& pl, int bits_lo, int* hbm_passes) {
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = lane(ctx).stream;
   if (pl.np == 0) return DBSP_OK;
   const u32 ntiles = (u32)((n + RS_TILE - 1) / RS_TILE);
   BufP aux;
@@ -558,7 +558,7 @@ int32_t run_chunks(Ctx* ctx, Bufs& B, int& cur, u64 n, int bits_total, int bits_
   MPairPtrs out{B.k0[cur ^ 1], B.k1[cur ^ 1], B.id[cur ^ 1], B.bid[cur ^ 1]};
   {
     ProfScope ps(ctx, KID_CHUNK_SORT, n * (u64)(2 * (8 * W + 4) + (BID ? 2 : 0)));
-    k_chunk_sort<W, BID><<<nwin, CsCfg<W>::THREADS, SMEM, ctx->stream>>>(in, out, n, bits_total, bits_lo, bshift, fail);
+    k_chunk_sort<W, BID><<<nwin, CsCfg<W>::THREADS, SMEM, lane(ctx).stream>>>(in, out, n, bits_total, bits_lo, bshift, fail);
   }
   LAUNCH_COUNT(ctx);
   cur ^= 1;
@@ -578,7 +578,7 @@ void lsd_passes(PassList& pl, int bits_total) {
 template <int W>
 int32_t sort_impl(Ctx* ctx, Bufs& B, u64 n, int bits_lo, int bits_hi, int presorted_top_bits, bool force_lsd, unsigned long long* fail,
                   int* cur_out, int* hbm_passes) {
-  cudaStream_t st = ctx->stream;
+  cudaStream_t st = lane(ctx).stream;
   const int bits_total = W == 1 ? bits_lo : bits_lo + bits_hi;
   int cur = 0;
   PassList pl;

@@ -48,7 +48,7 @@ class Runtime(Backend):
     name = "cuda"
 
     def __init__(self, device: int = 0):
-        super().__init__(CApi(load_library(), "dbsp_"), device)
+        super().__init__(CApi(load_library(), "dbsp_", require_grouped=True), device)
 
     @property
     def stream_ptr(self) -> int:

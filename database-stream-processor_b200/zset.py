@@ -19,7 +19,7 @@ from typing import Iterable, Sequence
 import numpy as np
 
 from . import _capi as capi
-from ._capi import CApi, CExpr, CPred, CProj, CSchema, CSrc, as_u64, col_ptrs
+from ._capi import CApi, CExpr, CPred, CProj, CSchema, CSrc, CTableJob, as_u64, col_ptrs
 
 
 @dataclass(frozen=True)
@@ -600,6 +600,43 @@ class Backend:
         self.api.call("batch_from_upload", self.ctx, up.h, proj.c(), C.byref(out))
         return Batch(self, out.value, proj.schema)
 
+    def batches_from_tables(self, tables: Sequence) -> list[Batch]:
+        """flat_map_index of several raw tables in one call: `tables` holds
+        (table, proj) pairs, a table being ("host", cols, weights, None),
+        ("dev", ptrs, weights, n) or ("upload", Upload, None, None) as
+        `TableHandle` takes them.  Returns what `batch_from_table` /
+        `batch_from_upload` would return for each pair; the CUDA library runs
+        the tables side by side on its two execution lanes."""
+        if self.api._batches_from_tables is None:   # a library without the grouped calls: the single calls in turn
+            return [self.batch_from_upload(t[1], p) if t[0] == "upload"
+                    else self.batch_from_table(t[1], p, weights=t[2], n=t[3], on_device=(t[0] == "dev")) for t, p in tables]
+        k = len(tables)
+        jobs = (CTableJob * max(k, 1))()
+        keep = []   # host arrays and C structs must outlive the call
+        for i, ((kind, cols, w, n), proj) in enumerate(tables):
+            j = jobs[i]
+            j.proj = C.pointer(proj._c)
+            if kind == "upload":
+                j.upload = cols.h
+                continue
+            if kind == "host":
+                cols = [as_u64(c) for c in cols]
+                n = len(cols[0])
+                if w is not None:
+                    w = np.ascontiguousarray(np.asarray(w, dtype=np.int64))
+                    keep.append(w)
+                    w = w.ctypes.data
+            ptrs = col_ptrs(cols)
+            keep.append((cols, ptrs))
+            j.cols = C.cast(ptrs, C.c_void_p)
+            j.weights = w
+            j.n = n
+            j.n_cols = len(cols)
+            j.on_device = int(kind == "dev")
+        outs = (C.c_void_p * max(k, 1))()
+        self.api.call("batches_from_tables", self.ctx, k, jobs, outs)
+        return [Batch(self, outs[i], tables[i][1].schema) for i in range(k)]
+
     def proj_table_mask(self, proj: Proj) -> int:
         return int(self.api._proj_table_mask(proj.c()))
 
@@ -653,6 +690,20 @@ class Backend:
     def join_delta_trace(self, delta: Batch, trace: Spine, proj: Proj, delta_is_left=True) -> Batch:
         out = self._out()
         self.api.call("join_delta_trace", self.ctx, delta.h, trace.h, proj.c(), int(delta_is_left), C.byref(out))
+        return Batch(self, out.value, proj.schema)
+
+    def join_step(self, dl: Batch, dr: Batch, lt: Spine, rt: Spine, proj: Proj) -> Batch:
+        """One step of the incremental join (operator/join.rs:180-292):
+        rt.insert(dr); o1 = dl |x| rt; o2 = dr |x| lt; lt.insert(dl); o1 + o2.
+        The CUDA library runs the two halves side by side."""
+        if self.api._join_step is None:   # a library without the grouped calls: the single calls in turn
+            rt.insert(dr)
+            o1 = self.join_delta_trace(dl, rt, proj, delta_is_left=True)
+            o2 = self.join_delta_trace(dr, lt, proj, delta_is_left=False)
+            lt.insert(dl)
+            return self.merge(o1, o2)
+        out = self._out()
+        self.api.call("join_step", self.ctx, dl.h, dr.h, lt.h, rt.h, proj.c(), C.byref(out))
         return Batch(self, out.value, proj.schema)
 
     def join_batches(self, left: Batch, right: Batch, proj: Proj) -> Batch:

@@ -137,7 +137,7 @@ const char* dbsp_last_error(void);
  * since the last reset (bench.py's gpu_launches / e2e byte counts). */
 int32_t dbsp_ctx_stats(dbsp_ctx* ctx, uint64_t* kernel_launches,
                        uint64_t* h2d_bytes, uint64_t* d2h_bytes, int32_t reset);
-/* Optional per-kernel timing (CUDA events on the context's stream around the
+/* Optional per-kernel timing (CUDA events on the stream of the execution lane that runs the
  * library's own kernels).  enable == 1 starts a fresh collection, enable == 2
  * pauses it (what was collected stays readable, nothing more is recorded —
  * a sampling window inside a longer timed region), enable == 0 ends it.  _read
@@ -149,7 +149,9 @@ int32_t dbsp_ctx_profile_read(dbsp_ctx* ctx, int32_t kernel_id, char* name32,
                               uint64_t* launches, double* ms,
                               uint64_t* alg_bytes);
 /* CUDA stream the context launches on (cudaStream_t as void*), so a host
- * can order its own work / CUDA events on it. */
+ * can order its own work / CUDA events on it.  This is execution lane 0; the
+ * work a grouped call runs on lane 1 is joined back into it before the call
+ * returns. */
 void* dbsp_ctx_stream(dbsp_ctx* ctx);
 
 /* ---- batches -------------------------------------------------------- */
@@ -184,6 +186,24 @@ int32_t dbsp_upload_begin(dbsp_ctx* ctx, const uint64_t* const* cols,
 int32_t dbsp_batch_from_upload(dbsp_ctx* ctx, dbsp_upload* up,
                                const dbsp_proj* proj, dbsp_batch** out);
 int32_t dbsp_upload_free(dbsp_upload* up);
+/* flat_map_index of k raw tables in one call.  Each job is either a table of
+ * columns (`upload` NULL; cols / weights / n / n_cols / on_device as for
+ * dbsp_batch_from_table) or an upload (the other fields are ignored).  outs[i]
+ * is the batch dbsp_batch_from_table / dbsp_batch_from_upload would return for
+ * jobs[i].  With k >= 2 the jobs are spread over the context's two execution
+ * lanes (DESIGN.md §3) and run side by side; with k == 1 the job runs inline.
+ * On failure no batch is returned. */
+typedef struct dbsp_table_job {
+  const uint64_t* const* cols;
+  const int64_t* weights;
+  uint64_t n;
+  dbsp_upload* upload;
+  const dbsp_proj* proj;
+  uint32_t n_cols;
+  int32_t on_device;
+} dbsp_table_job;
+int32_t dbsp_batches_from_tables(dbsp_ctx* ctx, uint32_t k,
+                                 const dbsp_table_job* jobs, dbsp_batch** outs);
 /* Columns of the table a projection reads (bit l = SRC_LVAL idx l). */
 uint32_t dbsp_proj_table_mask(const dbsp_proj* proj);
 int32_t dbsp_batch_empty(dbsp_ctx* ctx, const dbsp_schema* schema,
@@ -321,6 +341,16 @@ int32_t dbsp_spine_load(dbsp_ctx* ctx, const char* path, dbsp_spine** out);
 int32_t dbsp_join_delta_trace(dbsp_ctx* ctx, const dbsp_batch* delta,
                               const dbsp_spine* trace, const dbsp_proj* proj,
                               int32_t delta_is_left, dbsp_batch** out);
+/* One step of the incremental join operator (join.rs:180-292):
+ *   insert(right_trace, d_right); o1 = d_left |x| right_trace;
+ *   o2 = d_right |x| left_trace (flipped, = z^-1 of the left integral);
+ *   insert(left_trace, d_left); out = o1 + o2.
+ * The two halves run side by side on the context's two execution lanes; the
+ * result and both traces equal those of that sequence of calls. */
+int32_t dbsp_join_step(dbsp_ctx* ctx, const dbsp_batch* d_left,
+                       const dbsp_batch* d_right, dbsp_spine* left_trace,
+                       dbsp_spine* right_trace, const dbsp_proj* proj,
+                       dbsp_batch** out);
 /* Join::eval (join.rs:436-473): stateless batch x batch. */
 int32_t dbsp_join_batches(dbsp_ctx* ctx, const dbsp_batch* left,
                           const dbsp_batch* right, const dbsp_proj* proj,
